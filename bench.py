@@ -5,7 +5,7 @@
 One "step" = one evaluation of GpPredictor.logLikelihoodWithDerivatives (gp/regression/GpPredictor.scala:60-80)
 with nParams = D+2 = 10 on the synthetic C2 workload of SURVEY.md 8(d) (seed 2, X ~ U(0,1)^{8192x8}).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 * value  : evals/s with X, y resident in HBM (gpk_gp_nll_grad_dev), CUDA-event timed, max over ranks.
 * e2e    : same metric through the public host API (GpPredictor.logLikelihoodWithDerivatives) with pinned
@@ -15,6 +15,9 @@ with nParams = D+2 = 10 on the synthetic C2 workload of SURVEY.md 8(d) (seed 2, 
 * roofline: the Cholesky trailing update (SYRK on DMMA) timed alone against a live cuBLAS Dgemm peak.
 * cpu_baseline / --impl reference: the oracle's LAPACK-backed port on the box's host cores (the Scala
   reference needs a JVM, absent here -- see DESIGN.md).
+* --dump-outputs DIR: after the timed steps, what the last timed step returned, as DIR/ll.npy (N,) and DIR/grad.npy
+  (N, nparams) in float64, one row per rank.  The inputs are seeded, so two builds run with the same arguments can be
+  compared output for output.
 """
 import argparse
 import json
@@ -45,7 +48,13 @@ def parse():
     ap.add_argument("--n", type=int, default=N_TRAIN, help="(debug only) problem size; the reported config is n=8192")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-sharded", action="store_true", help="skip the C4 / C5 sharded record (debug)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's (ll, grad) to DIR/ll.npy, DIR/grad.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "gpk":
+        ap.error("--dump-outputs writes the outputs of the gpk path only")
+    return args
 
 
 def config(n, n_gpus):
@@ -416,6 +425,14 @@ def syrk_traffic(nn, kk):
     return {"traffic": None}
 
 
+def dump_outputs(path, res):
+    """res: (ranks, 1 + nparams) rows of gpk_gp_nll_grad_dev's output (ll, grad) -> path/ll.npy, path/grad.npy (float64)."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "ll.npy"), np.ascontiguousarray(res[:, 0], dtype=np.float64))
+    np.save(os.path.join(path, "grad.npy"), np.ascontiguousarray(res[:, 1:], dtype=np.float64))
+
+
 def run_gpk(args):
     import numpy as np
     import torch
@@ -483,6 +500,13 @@ def run_gpk(args):
     clocks = sampler.stop() if rank == 0 else None
     assert int(dinfo.item()) == 0, "factorisation failed"
     res_dev = dout.cpu().numpy().copy()
+    if args.dump_outputs:
+        rows = [dout]
+        if dist is not None:
+            rows = [torch.empty_like(dout) for _ in range(world)]
+            dist.all_gather(rows, dout)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, torch.stack(rows).cpu().numpy())
 
     # ---- e2e: public host API, pinned host buffers, H2D + D2H inside the timed region -----------------
     Xp = torch.from_numpy(np.asfortranarray(X).T.copy()).pin_memory()
