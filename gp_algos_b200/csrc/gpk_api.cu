@@ -114,11 +114,10 @@ int gpk_create(gpk_handle* out, int device, void* stream) {
     cudaDeviceGetStreamPriorityRange(&least, &greatest);
     cudaStreamGetPriority(h->stream, &mainprio);
     // numerically lower = more urgent; [greatest, least] is e.g. [-5, 0]
-    // three levels below the main stream when the device has them: side (fork/join of the recursion, near-critical panels),
-    // mid (the trailing update when right-hand sides / consumers ride along at the lowest level), pipe (lowest)
+    // below the main stream: side (fork/join of the recursion, near-critical panels) two levels above pipe (lowest) when the
+    // device has that many levels, else one level or none
     const bool wide = least - 2 > greatest && mainprio < least - 2;
     const int sideprio = wide ? least - 2 : ((mainprio < least && least - 1 >= greatest) ? least - 1 : least);
-    const int midprio = wide ? least - 1 : least;
     h->prio_main = mainprio; h->prio_side = sideprio; h->prio_pipe = least;
     const char* gm = getenv("GPK_GRAPH");
     const char* tr = getenv("GPK_TRACE");
@@ -129,8 +128,6 @@ int gpk_create(gpk_handle* out, int device, void* stream) {
         if (cudaStreamCreateWithPriority(&h->pipe[i], cudaStreamNonBlocking, least) != cudaSuccess) { delete h; return GPK_ECUDA; }
     for (int i = 0; i < GPK_NGROUP - 1; ++i)
         if (cudaStreamCreateWithPriority(&h->grp[i], cudaStreamNonBlocking, mainprio) != cudaSuccess) { delete h; return GPK_ECUDA; }
-    if (cudaStreamCreateWithPriority(&h->mid, cudaStreamNonBlocking, midprio) != cudaSuccess) { delete h; return GPK_ECUDA; }
-    h->prio_mid = midprio;
     for (int i = 0; i < GPK_NEVENTS; ++i)
         if (cudaEventCreateWithFlags(&h->evpool[i], cudaEventDisableTiming) != cudaSuccess) { delete h; return GPK_ECUDA; }
     *out = h;
@@ -142,14 +139,12 @@ int gpk_destroy(gpk_handle h) {
     cudaSetDevice(h->device);
     cudaStreamSynchronize(h->stream);
     gpk_graph_drop_all(h);
-    if (h->part) { cudaDeviceSynchronize(); gpk_partition_destroy(h->part); h->part = nullptr; }
     for (int i = 0; i < GPK_NSIDE; ++i)
         if (h->side[i]) { cudaStreamSynchronize(h->side[i]); cudaStreamDestroy(h->side[i]); }
     for (int i = 0; i < GPK_NPIPE; ++i)
         if (h->pipe[i]) { cudaStreamSynchronize(h->pipe[i]); cudaStreamDestroy(h->pipe[i]); }
     for (int i = 0; i < GPK_NGROUP - 1; ++i)
         if (h->grp[i]) { cudaStreamSynchronize(h->grp[i]); cudaStreamDestroy(h->grp[i]); }
-    if (h->mid) { cudaStreamSynchronize(h->mid); cudaStreamDestroy(h->mid); }
     for (int i = 0; i < GPK_NARENA; ++i)
         if (h->arena[i]) cudaFree(h->arena[i]);
     if (h->h_pinned) cudaFreeHost(h->h_pinned);

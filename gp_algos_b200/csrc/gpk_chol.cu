@@ -63,11 +63,6 @@ int pipe_min() {     // smallest padded N that takes the pipelined driver (0 dis
 int potrf_nb(int N);
 int potrf_nb_max();
 bool potrf_nb_forced();
-int mid_for_riders() {   // GPK_MID_STREAM=1: with riders, the trailing update runs one priority level above them (no gain measured)
-    static int v = -1;
-    if (v < 0) { const char* e = getenv("GPK_MID_STREAM"); v = e ? atoi(e) : 0; }
-    return v;
-}
 
 int batch_group_min() {   // smallest batch that is split into GPK_NGROUP concurrent groups (0 or less: never)
     static int v = -1;
@@ -436,41 +431,6 @@ int gpk_potrf_inv_pipelined(gpk_handle h, double* A, double* Li, double* Kinv, d
 }
 
 // ------------------------------------------------------------------------------------------------------------------
-// Runs the enclosed driver on the SM partition when there is one: the handle's stream becomes the partition's spine stream
-// (which first waits for everything queued on the caller's stream), the recursion's fork/join streams become the spine
-// partition's; finish() (or the destructor, on an error path) puts the handle back and makes the caller's stream wait.
-struct PartitionScope {
-    gpk_handle h;
-    gpk_partition* p = nullptr;
-    bool on = false;
-    cudaStream_t outer = nullptr;
-    cudaStream_t saved_side[GPK_NSIDE];
-    PartitionScope(gpk_handle h_, int N) : h(h_) {
-        if (!gpk_partition_active(h, N, &p)) return;
-        outer = h->stream;
-        cudaEvent_t e = next_event(h);
-        if (cudaEventRecord(e, outer) != cudaSuccess || cudaStreamWaitEvent(gpk_partition_stream(p, 0, 0), e, 0) != cudaSuccess) {
-            cudaGetLastError();
-            return;
-        }
-        for (int i = 0; i < GPK_NSIDE; ++i) { saved_side[i] = h->side[i]; h->side[i] = gpk_partition_stream(p, 1, i); }
-        h->stream = gpk_partition_stream(p, 0, 0);
-        on = true;
-    }
-    int finish() {
-        if (!on) return GPK_OK;
-        on = false;
-        cudaStream_t spine = h->stream;
-        h->stream = outer;
-        for (int i = 0; i < GPK_NSIDE; ++i) h->side[i] = saved_side[i];
-        cudaEvent_t e = next_event(h);
-        GPK_CUDA(h, cudaEventRecord(e, spine));
-        GPK_CUDA(h, cudaStreamWaitEvent(outer, e, 0));
-        return GPK_OK;
-    }
-    ~PartitionScope() { finish(); }
-};
-
 // Factor-only look-ahead driver (gpk_potrf_factor / gpk_potrf_factor_solve).  Without the inverse rows and the K^-1
 // accumulation there are only n^3/3 flops of bulk work to hide the serial spine behind, so the spine itself is cut to what
 // the NEXT diagonal block needs: per step k the handle's stream runs
@@ -519,16 +479,7 @@ int potrf_factor_pipelined(gpk_handle h, double* A, double* Li, double* T, int N
     auto bs = [&](int k) { return k * nbk < N ? k * nbk : N; };
     GPK_CUDA(h, cudaMemsetAsync(info_dev, 0, sizeof(int), h->stream));
     Ctx c{h, N, N, 1, info_dev, 1, (int64_t)N * N, 0, 0};
-    // (GPK_MID_STREAM=1: with riders on the lowest level the trailing update moves one level up -- the spine waits for its
-    // column-first piece, evG, 0.35-0.5 ms per step against 0.175 ms alone, profiles/r02_ep_refactor_trace.log; measured: no gain)
-    cudaStream_t M = h->stream, S = (rhsB && mid_for_riders()) ? h->mid : h->pipe[0], S1 = h->side[GPK_NSIDE - 1], R = h->pipe[1];
-    // SM partition (gpk_part.cu): the spine -- this function's launches on M and the fork/join streams of the diagonal-block
-    // recursion -- runs on SMs of its own, the bulk streams on the others; the caller's stream waits at both ends
-    PartitionScope part(h, N);
-    if (part.on) {
-        M = h->stream;                                    // = the partition's spine stream (swapped in by the scope)
-        S = gpk_partition_stream(part.p, 3, 0); S1 = gpk_partition_stream(part.p, 2, 0); R = gpk_partition_stream(part.p, 3, 1);
-    }
+    cudaStream_t M = h->stream, S = h->pipe[0], S1 = h->side[GPK_NSIDE - 1], R = h->pipe[1];
     cudaEvent_t ev0 = next_event(h);
     GPK_CUDA(h, cudaEventRecord(ev0, M));
     GPK_CUDA(h, cudaStreamWaitEvent(S, ev0, 0));
@@ -636,7 +587,7 @@ int potrf_factor_pipelined(gpk_handle h, double* A, double* Li, double* T, int N
         GPK_CUDA(h, cudaStreamWaitEvent(M, e3, 0));
     }
     tr.dump();
-    return part.finish();
+    return GPK_OK;
 }
 
 }  // namespace
@@ -746,12 +697,4 @@ int gpk_lauum_lower(gpk_handle h, const double* Li, double* Kinv, int N, int bat
     g.R = N; g.S = N; g.K = N; g.kb_r = 1; g.kb_s = 1; g.tri_out = 1;
     g.batch = batch; g.strideP = g.strideQ = g.strideD = (int64_t)N * N;
     return gpk_gemm(h, g);
-}
-
-bool gpk_partition_active(gpk_handle h, int N, gpk_partition** out) {
-    static int min_n = -1;
-    if (min_n < 0) { const char* e = getenv("GPK_PARTITION_MIN_N"); min_n = e ? atoi(e) : 2048; }
-    *out = nullptr;
-    if (h->cap || N < min_n || h->stream != h->main_stream) return false;
-    return gpk_partition_get(h, out) == 1;
 }

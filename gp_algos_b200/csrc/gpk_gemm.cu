@@ -8,7 +8,7 @@
 // DMMA and DFMA both peak at 37.1 TFLOP/s; DMMA needs 4x fewer shared-memory operand bytes per flop, which is what lets
 // a small CTA tile run pipe-bound.
 //
-// Default layout (SmallTile): 64 x 64 x 16 CTA tile, 128 threads = 4 warps as 2 (r) x 2 (s), each warp owning a 32 x 32
+// One layout (SmallTile): 64 x 64 x 16 CTA tile, 128 threads = 4 warps as 2 (r) x 2 (s), each warp owning a 32 x 32
 // sub-tile = 4 x 4 DMMA accumulators; 3 CTAs per SM (60 KB of shared memory each), which beat every larger tile shape
 // (profiles/r01_tile_configs.txt).  Operands are staged global -> shared with 16-byte cp.async (LDGSTS) through a 3-stage
 // ring; shared rows are padded by 4 doubles so that the 8-byte fragment reads of a half-warp (4 k x 4 rows) hit 16 distinct
@@ -16,8 +16,6 @@
 // the first DMMA group of each k-step.  Measured: 32.5 TFLOP/s on the SYRK of n = k = 4096 (91.7 % of cuBLAS Dgemm), DMMA
 // pipe 95 % of active cycles (profiles/r01_ncu_summary_v3.txt).
 #include "gpk_internal.cuh"
-
-#include <stdlib.h>
 
 namespace {
 
@@ -41,9 +39,6 @@ __device__ __forceinline__ void dmma(double& c0, double& c1, double a, double b)
 }
 
 // Tile configuration: WR x WS warps, each owning a (BI*8) x (BJ*8) sub-tile.
-//   Big  : 2 x 4 warps, 8 x 4 blocks -> 128 x 128 CTA tile, 256 threads, 1 CTA/SM   (throughput)
-//   Small: 2 x 2 warps, 4 x 4 blocks ->  64 x  64 CTA tile, 128 threads, 2 CTAs/SM  (few-tile problems: spreads a
-//          128-tile over 4 SMs; one SM can only retire 0.25 TFLOP/s of FP64)
 template <int WR_, int WS_, int BI_, int BJ_, int STAGES_, int MINB_>
 struct TileCfg {
     static constexpr int WR = WR_, WS = WS_, BI = BI_, BJ = BJ_, STAGES = STAGES_;
@@ -54,9 +49,6 @@ struct TileCfg {
     static constexpr size_t SMEM = (size_t)STAGES * (P_STAGE + Q_STAGE) * sizeof(double);
     static constexpr int MIN_BLOCKS = MINB_;
 };
-using BigTile = TileCfg<2, 4, 8, 4, 4, 1>;
-using WideTile = TileCfg<4, 4, 4, 4, 4, 1>;    // 128 x 128 tile on 16 warps of 32 x 32 (4 warps per scheduler)
-using MidTile = TileCfg<2, 2, 8, 4, 3, 2>;     // 128 x 64 tile, 4 warps of 64 x 32, 2 CTAs per SM
 using SmallTile = TileCfg<2, 2, 4, 4, 3, 3>;   // 3 stages x 20 KB = 60 KB -> 3 CTAs (12 warps) per SM
 
 // One CTA tile: acc += sum over nk k-chunks (of TK) starting at kbeg of P(r0.., k) Q(s0.., k).  Called by every thread of the
@@ -202,121 +194,9 @@ __global__ void __launch_bounds__(Cfg::NT, Cfg::MIN_BLOCKS) gemm_f64_dmma_kernel
     tile_epilogue<Cfg>(g, D, Cin, r0, s0, acc);
 }
 
-// ---------------------------------------------------------------------------------------------------------------------
-// Stream-K variant for the large uniform GEMMs (the Cholesky trailing update): a launch of T equal tiles on G = 3 x SMs
-// resident CTAs leaves the last T mod G tiles' wave partly empty (SYRK n = k = 4096: 2080 tiles on 444 slots = 4.68 waves,
-// 6.8 % idle).  Here the grid is exactly G persistent CTAs: the first T - (G + T mod G) tiles are handed out whole
-// (data-parallel waves), and the k-iterations of the remaining G + (T mod G) tiles are cut into G equal contiguous ranges,
-// so every CTA finishes at the same time.  A CTA whose range covers only part of a tile writes its raw accumulators to a
-// workspace slot; a second small kernel adds the partials of each split tile in ascending-k order (deterministic: no
-// atomics, no waiting between CTAs) and applies the epilogue.
-// ---------------------------------------------------------------------------------------------------------------------
-struct SkPlan {
-    int G, nk, dp_tiles, sk_tiles, nT;   // nT: tiles per side of a tri_out problem
-    long long I;                         // k-iterations of the stream-K region = sk_tiles * nk
-    double* ws;                          // 2 G slots of TR x TS doubles
-};
-
-template <class Cfg>
-__device__ __forceinline__ void sk_tile_origin(const GemmDesc& g, const SkPlan& sk, int t, int& r0, int& s0) {
-    constexpr int TR = Cfg::TR, TS = Cfg::TS;
-    if (g.tri_out) {
-        // lower tiles (ts >= tr) column by column: column tr starts at tr nT - tr (tr - 1) / 2
-        const int nT = sk.nT;
-        const double b = 2.0 * nT + 1.0;
-        int tr = (int)((b - sqrt(b * b - 8.0 * t)) * 0.5);
-        tr = max(0, min(tr, nT - 1));
-        while (tr > 0 && tr * nT - tr * (tr - 1) / 2 > t) --tr;
-        while ((tr + 1) * nT - (tr + 1) * tr / 2 <= t) ++tr;
-        const int ts = tr + (t - (tr * nT - tr * (tr - 1) / 2));
-        r0 = tr * TR; s0 = ts * TS;
-    } else {
-        const int tilesS = g.S / TS, tilesR = g.R / TR;
-        const int group = t / (GROUP_S * tilesR);
-        const int first_s = group * GROUP_S;
-        const int gs = min(GROUP_S, tilesS - first_s);
-        const int within = t - group * GROUP_S * tilesR;
-        r0 = (within / gs) * TR; s0 = (first_s + within % gs) * TS;
-    }
-}
-
 template <bool PK, bool QK, class Cfg>
-__global__ void __launch_bounds__(Cfg::NT, Cfg::MIN_BLOCKS) gemm_f64_dmma_sk_kernel(const GemmDesc g, const SkPlan sk) {
-    constexpr int BI = Cfg::BI, BJ = Cfg::BJ, NT = Cfg::NT;
-    extern __shared__ __align__(16) double smem[];
-    const int bid = blockIdx.x;
-    double acc[BI][BJ][2];
-    auto zero = [&]() {
-#pragma unroll
-        for (int i = 0; i < BI; ++i)
-#pragma unroll
-            for (int j = 0; j < BJ; ++j) acc[i][j][0] = acc[i][j][1] = 0.0;
-    };
-    int r0, s0;
-    for (int t = bid; t < sk.dp_tiles; t += sk.G) {                 // whole tiles
-        sk_tile_origin<Cfg>(g, sk, t, r0, s0);
-        zero();
-        tile_mainloop<PK, QK, Cfg>(g, g.P, g.Q, r0, s0, 0, sk.nk, smem, acc);
-        tile_epilogue<Cfg>(g, g.D, g.Cin, r0, s0, acc);
-        __syncthreads();                                            // the ring is refilled by the next tile's prologue
-    }
-    const long long a = (long long)bid * sk.I / sk.G, b = (long long)(bid + 1) * sk.I / sk.G;
-    for (long long it = a; it < b;) {                               // this CTA's share of the stream-K region
-        const int t = (int)(it / sk.nk), k0 = (int)(it - (long long)t * sk.nk);
-        const int k1 = (int)min((long long)sk.nk, k0 + (b - it));
-        sk_tile_origin<Cfg>(g, sk, sk.dp_tiles + t, r0, s0);
-        zero();
-        tile_mainloop<PK, QK, Cfg>(g, g.P, g.Q, r0, s0, k0 * TK, k1 - k0, smem, acc);
-        if (k0 == 0 && k1 == sk.nk) {
-            tile_epilogue<Cfg>(g, g.D, g.Cin, r0, s0, acc);
-        } else {                                                    // partial: raw accumulators, fragment-major (coalesced)
-            double2* w = reinterpret_cast<double2*>(sk.ws) + (size_t)(2 * bid + (it == a ? 0 : 1)) * (BI * BJ * NT);
-#pragma unroll
-            for (int i = 0; i < BI; ++i)
-#pragma unroll
-                for (int j = 0; j < BJ; ++j) w[(i * BJ + j) * NT + threadIdx.x] = make_double2(acc[i][j][0], acc[i][j][1]);
-        }
-        __syncthreads();
-        it += k1 - k0;
-    }
-}
-
-// one CTA per tile of the stream-K region: tiles that were split get their partials summed (ascending k) and the epilogue
-template <class Cfg>
-__global__ void __launch_bounds__(Cfg::NT) gemm_sk_fixup_kernel(const GemmDesc g, const SkPlan sk) {
-    constexpr int BI = Cfg::BI, BJ = Cfg::BJ, NT = Cfg::NT;
-    const int t = blockIdx.x;
-    const long long first = (long long)t * sk.nk, last = first + sk.nk - 1;
-    auto lo = [&](int c) { return (long long)c * sk.I / sk.G; };
-    int c = (int)min((long long)sk.G - 1, first * sk.G / sk.I);
-    while (c > 0 && lo(c) > first) --c;
-    while (c + 1 < sk.G && lo(c + 1) <= first) ++c;
-    if (lo(c + 1) > last) return;                                   // one CTA did the whole tile and its epilogue
-    double acc[BI][BJ][2];
-#pragma unroll
-    for (int i = 0; i < BI; ++i)
-#pragma unroll
-        for (int j = 0; j < BJ; ++j) acc[i][j][0] = acc[i][j][1] = 0.0;
-    for (; c < sk.G && lo(c) <= last; ++c) {
-        if (lo(c + 1) <= first) continue;                           // empty range
-        const long long seg = max(lo(c), first);
-        const double2* w = reinterpret_cast<const double2*>(sk.ws) + (size_t)(2 * c + (seg == lo(c) ? 0 : 1)) * (BI * BJ * NT);
-#pragma unroll
-        for (int i = 0; i < BI; ++i)
-#pragma unroll
-            for (int j = 0; j < BJ; ++j) {
-                const double2 v = w[(i * BJ + j) * NT + threadIdx.x];
-                acc[i][j][0] += v.x; acc[i][j][1] += v.y;
-            }
-    }
-    int r0, s0;
-    sk_tile_origin<Cfg>(g, sk, sk.dp_tiles + t, r0, s0);
-    tile_epilogue<Cfg>(g, g.D, g.Cin, r0, s0, acc);
-}
-
-template <bool PK, bool QK, class Cfg>
-int launch(gpk_handle h, const GemmDesc& g, int cfg_id) {
-    const unsigned bit = 1u << (12 + cfg_id * 4 + (PK ? 2 : 0) + (QK ? 1 : 0));
+int launch(gpk_handle h, const GemmDesc& g) {
+    const unsigned bit = 1u << (12 + (PK ? 2 : 0) + (QK ? 1 : 0));
     if (!(h->func_cfg & bit)) {
         GPK_CUDA(h, cudaFuncSetAttribute(gemm_f64_dmma_kernel<PK, QK, Cfg>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          (int)Cfg::SMEM));
@@ -329,106 +209,17 @@ int launch(gpk_handle h, const GemmDesc& g, int cfg_id) {
 }
 
 template <class Cfg>
-int dispatch(gpk_handle h, const GemmDesc& g, int cfg_id) {
-    if (g.p_kcontig) return g.q_kcontig ? launch<true, true, Cfg>(h, g, cfg_id) : launch<true, false, Cfg>(h, g, cfg_id);
-    return g.q_kcontig ? launch<false, true, Cfg>(h, g, cfg_id) : launch<false, false, Cfg>(h, g, cfg_id);
-}
-
-// GPK_STREAMK=1 enables the stream-K path.  OFF by default -- measured on B200 (profiles/r02_streamk.log): the isolated SYRK
-// n = k = 4096 gains 0.8 % (2.113 -> 2.097 ms), launches with k = 512 lose 11 % (1.016 -> 1.143 ms), and the whole evaluation
-// at n = 8192 loses 10 % (17.40 -> 19.14 ms): persistent CTAs hold every SM slot for the whole launch, so the look-ahead
-// driver's high-priority spine kernels can no longer slip in between the bulk update's short CTAs.
-int stream_k_mode() {   // read at every launch (a getenv, ~50 ns) so that a test can switch it inside one process
-    const char* e = getenv("GPK_STREAMK");
-    return e ? atoi(e) : 0;
-}
-
-// which workspace slot a stream owns: the handle's stream and the three bulk streams of the look-ahead driver; -1 otherwise
-int sk_slot(gpk_handle h) {
-    if (h->stream == h->main_stream) return 0;
-    for (int i = 0; i < GPK_NPIPE; ++i) if (h->stream == h->pipe[i]) return 1 + i;
-    return -1;
-}
-
-template <bool PK, bool QK>
-int launch_sk(gpk_handle h, const GemmDesc& g, const SkPlan& sk) {
-    using Cfg = SmallTile;
-    const unsigned bit = 1u << (28 + (PK ? 2 : 0) + (QK ? 1 : 0));
-    if (!(h->func_cfg & bit)) {
-        GPK_CUDA(h, cudaFuncSetAttribute(gemm_f64_dmma_sk_kernel<PK, QK, Cfg>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         (int)Cfg::SMEM));
-        h->func_cfg |= bit;
-    }
-    gemm_f64_dmma_sk_kernel<PK, QK, Cfg><<<sk.G, Cfg::NT, Cfg::SMEM, h->stream>>>(g, sk);
-    GPK_LAUNCH_CHECK(h);
-    gemm_sk_fixup_kernel<Cfg><<<sk.sk_tiles, Cfg::NT, 0, h->stream>>>(g, sk);
-    GPK_LAUNCH_CHECK(h);
-    return GPK_OK;
-}
-
-// returns 1 when the launch was taken by the stream-K path, 0 when the caller should use the plain kernel, < 0 on error
-int try_stream_k(gpk_handle h, const GemmDesc& g) {
-    using Cfg = SmallTile;
-    if (!stream_k_mode() || g.batch != 1 || g.kb_r || g.kb_s || g.ke_r || g.ke_s) return 0;
-    if (g.tri_out && g.R != g.S) return 0;
-    const int nk = g.K / TK;
-    const int G = 3 * h->num_sms;
-    const int tilesR = g.R / Cfg::TR, tilesS = g.S / Cfg::TS;
-    const long long T = g.tri_out ? (long long)tilesR * (tilesR + 1) / 2 : (long long)tilesR * tilesS;
-    if (nk < 16 || T < G || T % G == 0 || T > (1 << 24)) return 0;
-    const int waves_up = (int)((T + G - 1) / G);
-    if ((double)(waves_up * (long long)G - T) / ((double)waves_up * G) < 0.02) return 0;   // the tail already wastes < 2 %
-    const int slot = sk_slot(h);
-    if (slot < 0) return 0;
-    const size_t slot_bytes = (size_t)2 * G * Cfg::TR * Cfg::TS * sizeof(double);
-    char* ws = (char*)gpk_arena(h, ARENA_SK, slot_bytes * (1 + GPK_NPIPE));
-    if (!ws) return 0;                                              // (e.g. first use during graph capture)
-    SkPlan sk;
-    sk.G = G; sk.nk = nk; sk.nT = tilesR;
-    sk.sk_tiles = (int)(G + T % G);
-    sk.dp_tiles = (int)(T - sk.sk_tiles);
-    sk.I = (long long)sk.sk_tiles * nk;
-    sk.ws = (double*)(ws + slot_bytes * slot);
-    int rc;
-    if (g.p_kcontig) rc = g.q_kcontig ? launch_sk<true, true>(h, g, sk) : launch_sk<true, false>(h, g, sk);
-    else rc = g.q_kcontig ? launch_sk<false, true>(h, g, sk) : launch_sk<false, false>(h, g, sk);
-    return rc ? rc : 1;
-}
-
-int small_tile_threshold() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("GPK_SMALL_TILE_THRESHOLD");
-        // Measured on B200 (profiles/r01_tile_configs.txt): 64x64 tiles at 3 CTAs/SM beat the 128x128 (1 CTA/SM) and
-        // 128x64 (2 CTAs/SM) configurations at every size (SYRK n=k=4096: 31.2 vs 26.8 vs 29.1 TFLOP/s), so they are
-        // the default everywhere; the threshold stays as a tuning knob.
-        v = e ? atoi(e) : 0x7fffffff;
-    }
-    return v;
+int dispatch(gpk_handle h, const GemmDesc& g) {
+    if (g.p_kcontig) return g.q_kcontig ? launch<true, true, Cfg>(h, g) : launch<true, false, Cfg>(h, g);
+    return g.q_kcontig ? launch<false, true, Cfg>(h, g) : launch<false, false, Cfg>(h, g);
 }
 
 }  // namespace
 
 int gpk_gemm(gpk_handle h, const GemmDesc& g) {
     if (g.R <= 0 || g.S <= 0 || g.batch <= 0) return GPK_OK;
-    // (64-granular shapes are served by the 64 x 64 tile configuration only)
-    const bool small_only = (g.R % 128) || (g.S % 128);
     if (g.R % 64 || g.S % 64 || g.K % TK || (g.ldp & 1) || (g.ldq & 1) || (g.ldd & 1) ||
         ((uintptr_t)g.P & 15) || ((uintptr_t)g.Q & 15) || ((uintptr_t)g.D & 15) || (g.Cin && (((uintptr_t)g.Cin & 15) || (g.ldc & 1))))
         return gpk_set_error(h, GPK_EINVAL, "gpk_gemm: unaligned problem R=%d S=%d K=%d", g.R, g.S, g.K);
-    int64_t tiles = (int64_t)(g.R / 128) * (g.S / 128) * g.batch;
-    if (g.tri_out) tiles = (tiles + g.batch * (g.R / 128)) / 2;
-    if (g.cfg_hint == 1 && !small_only) return dispatch<BigTile>(h, g, 0);
-    if (g.cfg_hint == 2 && !small_only) return dispatch<WideTile>(h, g, 2);
-    if (g.cfg_hint == 3 && g.R % 128 == 0) return dispatch<MidTile>(h, g, 3);
-    if (small_only || tiles < small_tile_threshold()) {
-        const int sk = try_stream_k(h, g);
-        if (sk != 0) return sk < 0 ? sk : GPK_OK;
-        return dispatch<SmallTile>(h, g, 1);
-    }
-    static int big_kind = -1;
-    if (big_kind < 0) { const char* e = getenv("GPK_BIG_KIND"); big_kind = e ? atoi(e) : 0; }
-    if (big_kind == 1) return dispatch<WideTile>(h, g, 2);
-    if (big_kind == 2) return dispatch<MidTile>(h, g, 3);
-    return dispatch<BigTile>(h, g, 0);
+    return dispatch<SmallTile>(h, g);
 }

@@ -48,14 +48,12 @@ void gpk_capture_note(gpk_handle h) {
     for (int i = 0; i < GPK_NSIDE; ++i) if (h->stream == h->side[i]) cls = 1;
     for (int i = 0; i < GPK_NPIPE; ++i) if (h->stream == h->pipe[i]) cls = 2 + i;
     int prio = cls == 0 ? h->prio_main : cls == 1 ? h->prio_side : h->prio_pipe;
-    const bool on_mid = h->stream == h->mid;
     static int over[2 + GPK_NPIPE], have = -1;
     if (have < 0) {   // GPK_GRAPH_PRIO="main,side,pipe0,pipe1,pipe2" (tuning aid; the defaults measured best, profiles/r01_graph_sweep.log)
         const char* e = getenv("GPK_GRAPH_PRIO");
         have = e && sscanf(e, "%d,%d,%d,%d,%d", &over[0], &over[1], &over[2], &over[3], &over[4]) == 5;
     }
     if (have) prio = over[cls];
-    if (on_mid) prio = h->prio_mid;
     h->cap->nodes.emplace_back(deps[0], prio);
 }
 

@@ -24,8 +24,6 @@ struct gpk_handle_s {
     cudaStream_t side[GPK_NSIDE];
     cudaStream_t grp[GPK_NGROUP - 1];   // same priority as the main stream
     cudaStream_t pipe[GPK_NPIPE];   // lowest-priority streams of the pipelined factorisation (trailing updates; inverse rows; K^-1)
-    cudaStream_t mid;               // one level above pipe[]: the trailing update when consumers of the factor ride along on pipe[]
-    int prio_mid;
     cudaEvent_t evpool[GPK_NEVENTS];
     unsigned ev_next;
     // grow-only device arenas (A: factor / K^-1, B: L^-1, T: GEMM scratch, misc: small vectors)
@@ -47,18 +45,9 @@ struct gpk_handle_s {
     struct gpk_graph_slot* slots[3];   // cached graphs (gpk_graph.cu): GPK_SLOT_EVAL, GPK_SLOT_EP_SWEEP, GPK_SLOT_POTRF
     struct gpk_capture_log* cap;  // non-null while capturing: every kernel node with the priority of the stream it came from
     int prio_main, prio_side, prio_pipe;
-    struct gpk_partition* part;   // SM partition for the spine of the look-ahead factorisation (gpk_part.cu), created on first use
-    int part_state;               // 0 not tried, 1 ready, -1 unavailable / off
     int kernel_family;            // gpk_kernel_family: how (D, theta) arguments are interpreted
     char err[512];
 };
-// ---- SM partition (gpk_part.cu) ----
-int gpk_partition_get(gpk_handle h, struct gpk_partition** out);      // 1 when available
-void gpk_partition_destroy(struct gpk_partition* p);
-int gpk_partition_sms(const struct gpk_partition* p, int which);      // 0 spine, 1 bulk
-cudaStream_t gpk_partition_stream(const struct gpk_partition* p, int kind, int i);   // 0 spine, 1 spine side i, 2 bulk near-critical, 3 bulk i
-// does the factor-only look-ahead driver run partitioned for this size?  (not while a graph is being captured)
-bool gpk_partition_active(gpk_handle h, int N, struct gpk_partition** out);
 // ---- graph replay (gpk_graph.cu) ----
 #define GPK_NSLOTS 3
 enum { GPK_SLOT_EVAL = 0, GPK_SLOT_EP_SWEEP = 1, GPK_SLOT_POTRF = 2 };
@@ -73,7 +62,7 @@ int gpk_graph_run(gpk_handle h, int slot, const GraphKey& key, int eager_calls, 
     return gpk_graph_run_impl(h, slot, key, eager_calls, [](void* c) { return (*static_cast<F*>(c))(); }, &body, what);
 }
 
-enum { ARENA_A = 0, ARENA_B = 1, ARENA_T = 2, ARENA_MISC = 3, ARENA_X = 4, ARENA_IO = 5, ARENA_IO2 = 6, ARENA_IO3 = 7, ARENA_PP = 8, ARENA_INFO = 9, ARENA_GEMV = 10, ARENA_KINV = 11, ARENA_SK = 12, GPK_NARENA = 13 };
+enum { ARENA_A = 0, ARENA_B = 1, ARENA_T = 2, ARENA_MISC = 3, ARENA_X = 4, ARENA_IO = 5, ARENA_IO2 = 6, ARENA_IO3 = 7, ARENA_PP = 8, ARENA_INFO = 9, ARENA_GEMV = 10, ARENA_KINV = 11, GPK_NARENA = 12 };
 
 int gpk_set_error(gpk_handle h, int status, const char* fmt, ...);
 // returns device pointer to at least `bytes` bytes in arena `which` (contents undefined after growth)
@@ -126,7 +115,6 @@ struct GemmDesc {
     int tri_out;
     int kb_r, kb_s, ke_r, ke_s;
     int heavy_last;  // reverse tile order (heavy tiles are at high indices)
-    int cfg_hint;    // 0: default tile configuration; 1 / 2 / 3: 128x128 on 8 warps / 128x128 on 16 warps / 128x64, when the shape allows
 };
 static inline GemmDesc gemm_desc() {
     GemmDesc g;

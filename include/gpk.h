@@ -56,15 +56,12 @@ const char* gpk_version(void);
  * (tools/base_timing.py prints them; profiles/r02_base_timing.log). */
 int gpk_debug_base_timing(gpk_handle h, long long* stamps_host);
 /* Development aid: clock64() stamps of the EP site kernel on one synthetic 64-site block (tools/ep_site_timing.py).
- * chain 1..4: ep_sites_block_w with that GPK_EP_CHAIN; chain >= 10: ep_sites_block_p (the default kernel).
+ * chain 1: ep_sites_block_w (the reference kernel the tests compare against); chain >= 10: ep_sites_block_p (the default
+ * kernel); any other chain: GPK_EINVAL.
  * stamps_host must hold 14 * 64 + 1 = 897 entries: [0..319] five stamps per site of the (scalar) warp, [320] duration in ns of
  * one unstamped launch of the default kernel, [321..576] barrier arrival of four other warps per site, [577..896] phases of
  * tile warp 0 (the last two groups for chain >= 10 only). */
 int gpk_debug_ep_site_timing(gpk_handle h, int chain, long long* stamps_host);
-/* Opt-in SM partition for the spine of the factor-only look-ahead driver (GPK_PARTITION=1, GPK_SPINE_SMS; CUDA green contexts):
- * returns 1 and the two SM counts when the partition is up on this handle (creating it on first use), 0 when it is off or the
- * driver / device does not support it.  Measured and left off by default (DESIGN.md 7a). */
-int gpk_debug_partition(gpk_handle h, int* spine_sms, int* bulk_sms);
 /* Launch sequences that callers repeat verbatim are captured into CUDA graphs and replayed: the single-problem
  * gpk_gp_nll_grad[_dev] evaluation (an optimiser's objective, GpPredictor.scala:126-142; same buffers and shape, new
  * hyper-parameters through device memory) from its second call on, the device-resident factor-only Cholesky up to n = 4096

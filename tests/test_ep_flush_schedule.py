@@ -1,12 +1,13 @@
-"""The EP sweep's delayed flush in pairs of blocks (gp_algos_b200/csrc/gpk_ep.cu: ep_sweep_sites / ep_pair_flush, the default
-GPK_EP_LOOKAHEAD=2) as a bookkeeping model: every tile of Sigma0 that a later step reads must have received the update of
-every earlier block EXACTLY once by then -- whatever the number of blocks, padded size or folded schedule.  The piece list
-below restates ep_pair_flush (same order, same bounds); the model executes it in program order (it checks coverage, not the
+"""The EP sweep's delayed flush in pairs of blocks (gp_algos_b200/csrc/gpk_ep.cu: ep_sweep_sites / ep_pair_flush) as a
+bookkeeping model: every tile of Sigma0 that a later step reads must have received the update of
+every earlier block EXACTLY once by then -- whatever the number of blocks or padded size.  The piece list below restates
+ep_pair_flush (same order, same bounds; fold=False); the model executes it in program order (it checks coverage, not the
 stream dependencies) and counts, per 64 x 64 tile, which blocks' updates have been applied.
 
 What reads what (EpParameterEstimator.scala:44-61 in delayed-update form): apply(b) reads the CROSS of block b -- tile row b left
-of the diagonal and tile column b below it -- as of block b-1; in the folded schedule the site kernel of block b reads tile
-(b, b-1) as of block b-2 and that tile's block b-1 update arrives late (ep_late_tile)."""
+of the diagonal and tile column b below it -- as of block b-1.  fold=True models the folded schedule, which was measured no
+faster and removed from the library (DESIGN.md 7a): there the site kernel of block b read tile (b, b-1) as of block b-2 and
+that tile's block b-1 update arrived late, behind it."""
 import itertools
 
 import numpy as np

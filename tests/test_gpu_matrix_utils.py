@@ -204,27 +204,6 @@ def test_triangular_solves_blocked_substitution_large(n, m):
         assert np.allclose(got, want, rtol=1e-9, atol=1e-9 * np.abs(want).max())
 
 
-def test_cholesky_on_the_sm_partition(monkeypatch):
-    """GPK_PARTITION=1: the spine of the factor-only look-ahead driver on SMs of its own (CUDA green contexts, gpk_part.cu).
-    Same factor as on the ordinary streams; skipped where the driver cannot split the device."""
-    import ctypes as C
-    from gp_algos_b200 import _lib
-    X, y, th = orc.make_c2(n=2300, D=8, seed=5)
-    K = orc.fast_build_kernel_matrix(X, th)
-    L0 = MU.cholesky(K)
-    monkeypatch.setenv("GPK_PARTITION", "1")
-    monkeypatch.setenv("GPK_SPINE_SMS", "16")
-    h = _lib.Handle(0)
-    a, b = C.c_int(0), C.c_int(0)
-    if not h.lib.gpk_debug_partition(h.h, C.addressof(a), C.addressof(b)):
-        pytest.skip("no SM partition on this driver / device")
-    assert a.value >= 8 and b.value > a.value
-    L1 = MU.cholesky(K, handle=h)
-    L2 = MU.cholesky(K, handle=h)
-    assert np.array_equal(L1, L2)
-    assert np.allclose(L1, L0, rtol=1e-12, atol=1e-14)
-
-
 @pytest.mark.parametrize("n,lda", [(2048, 2048), (1500, 1504)])
 def test_potrf_lower_dev_graph_replay(n, lda):
     """The same buffers factored again: eager first, captured into a CUDA graph at the second call, replayed afterwards

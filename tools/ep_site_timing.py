@@ -6,7 +6,7 @@ import numpy as np
 from gp_algos_b200 import _lib
 h = _lib.default_handle()
 st = (C.c_longlong * 897)()
-for chain in (1, 2, 3, 4, 10):     # 10 = warp-specialised kernel (ep_sites_block_p, branch-free scalar update): loop-top stamps only
+for chain in (1, 10):     # 1 = reference kernel (ep_sites_block_w); 10 = warp-specialised kernel (ep_sites_block_p, branch-free scalar update): loop-top stamps only
     h.check(h.lib.gpk_debug_ep_site_timing(h.h, chain, C.addressof(st)))
     v = np.array(list(st)[:320], dtype=np.int64).reshape(64, 5)
     top, sc, dn, pub, bar = v.T

@@ -18,4 +18,4 @@ for _ in range(3):
     h.check(h.lib.gpk_syrk_lower_dev(h.h, P.data_ptr(), n, Cm.data_ptr(), n, n, k))
 e1.record(); torch.cuda.synchronize()
 ms = e0.elapsed_time(e1) / 3
-print(f"syrk n={n} k={k} GPK_STREAMK={os.environ.get('GPK_STREAMK', '0')}: {ms:.3f} ms  {n*n*k/ms*1e-9:.2f} TFLOP/s")
+print(f"syrk n={n} k={k}: {ms:.3f} ms  {n*n*k/ms*1e-9:.2f} TFLOP/s")
