@@ -108,6 +108,8 @@ def load():
         lib.gpk_gp_predict_batched.argtypes = [vp, ci, vp, ci, ci, _i64, _i64, vp, vp, vp, ci, _i64, _i64, ci, cd, vp, vp, vp, vp]
         lib.gpk_debug_base_timing.argtypes = [vp, vp]
         lib.gpk_debug_ep_site_timing.argtypes = [vp, C.c_int, vp]
+        lib.gpk_debug_gemm.argtypes = [vp, vp, _i64, _i64, vp, _i64, _i64, vp, _i64, _i64, vp, _i64, _i64,
+                                       ci, ci, ci, ci, cd, cd, ci, ci, ci]
         lib.gpk_mg_create.argtypes = [C.POINTER(vp), ci, vp]
         lib.gpk_mg_destroy.argtypes = [vp]
         lib.gpk_mg_last_error.argtypes = [vp]

@@ -223,3 +223,25 @@ int gpk_gemm(gpk_handle h, const GemmDesc& g) {
         return gpk_set_error(h, GPK_EINVAL, "gpk_gemm: unaligned problem R=%d S=%d K=%d", g.R, g.S, g.K);
     return dispatch<SmallTile>(h, g);
 }
+
+extern "C" int gpk_debug_gemm(gpk_handle h, const double* P, int64_t ldp, int64_t strideP, const double* Q, int64_t ldq,
+                              int64_t strideQ, double* D, int64_t ldd, int64_t strideD, const double* Cin, int64_t ldc,
+                              int64_t strideC, int R, int S, int K, int batch, double alpha, double beta, int p_kcontig,
+                              int q_kcontig, int flags) {
+    if (!h) return GPK_EINVAL;
+    if (flags & ~0x3f) return gpk_set_error(h, GPK_EINVAL, "gpk_debug_gemm: unknown flag bits 0x%x", flags);
+    GemmDesc g = gemm_desc();
+    g.P = P; g.ldp = ldp; g.strideP = strideP;
+    g.Q = Q; g.ldq = ldq; g.strideQ = strideQ;
+    g.D = D; g.ldd = ldd; g.strideD = strideD;
+    g.Cin = Cin; g.ldc = ldc; g.strideC = strideC;
+    g.R = R; g.S = S; g.K = K; g.batch = batch; g.alpha = alpha; g.beta = beta;
+    g.p_kcontig = p_kcontig != 0; g.q_kcontig = q_kcontig != 0;
+    g.tri_out = (flags & GPK_GEMM_TRI_OUT) != 0;
+    g.kb_r = (flags & GPK_GEMM_KB_R) != 0;
+    g.kb_s = (flags & GPK_GEMM_KB_S) != 0;
+    g.ke_r = (flags & GPK_GEMM_KE_R) != 0;
+    g.ke_s = (flags & GPK_GEMM_KE_S) != 0;
+    g.heavy_last = (flags & GPK_GEMM_HEAVY_LAST) != 0;
+    return gpk_gemm(h, g);
+}

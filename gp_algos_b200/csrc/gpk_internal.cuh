@@ -92,16 +92,17 @@ int gpk_finish_info(gpk_handle h);  // sync, read h->d_info[0], map to GPK_ENOTP
 static inline int gpk_pad(int n) { return (n + GPK_TILE - 1) / GPK_TILE * GPK_TILE; }
 
 // ---------------------------------------------------------------------------------------------
-// DMMA GEMM (gpk_gemm.cu).  Computes, for every 128x128 tile selected by `tri_out`,
+// DMMA GEMM (gpk_gemm.cu).  Computes, for every 64x64 tile (first row r0, first column s0) selected by `tri_out`,
 //     D(r,s) = alpha * sum_{k in [kbeg,kend)} P(r,k) * Q(s,k) + beta * Cin(r,s)
 // with D(r,s) stored at D[s + r*ldd] (s contiguous).  For a column-major C (M x N) this is D = C^t:
-// r is C's column index, s is C's row index.
+// r is C's column index, s is C's row index.  Cin may be null (no beta term, Cin never read) or alias D.
 //   p_kcontig: P(r,k) at P[k + r*ldp]   else P[r + k*ldp]
 //   q_kcontig: Q(s,k) at Q[k + s*ldq]   else Q[s + k*ldq]
 // k-range per tile (tile-granular exploitation of triangular operands):
-//   kbeg = max(kb_r ? r0 : 0, kb_s ? s0 : 0);  kend = min(K, ke_r ? r0+128 : K, ke_s ? s0+128 : K)
-// tri_out: only tiles with s0 >= r0 are computed (lower triangle of the column-major C).
-// R, S multiples of 128; K multiple of 16; pointers 16-byte aligned; ld's even.
+//   kbeg = max(kb_r ? r0 : 0, kb_s ? s0 : 0);  kend = min(K, ke_r ? r0+64 : K, ke_s ? s0+64 : K)
+// so a triangular operand must hold real zeros inside its diagonal 64-tile; beyond that tile nothing is read.
+// tri_out: only tiles with s0 >= r0 are computed (lower triangle of the column-major C); the other tiles of D are not written.
+// R, S multiples of 64; K multiple of 16; pointers 16-byte aligned; ld's even (gpk_gemm returns GPK_EINVAL otherwise).
 // ---------------------------------------------------------------------------------------------
 struct GemmDesc {
     const double* P; int64_t ldp; int64_t strideP;

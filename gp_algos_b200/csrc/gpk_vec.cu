@@ -234,7 +234,13 @@ int gpk_colwise_dot(gpk_handle h, const double* M, int64_t ld, int rows, int col
 
 int gpk_gemv(gpk_handle h, int trans, int m, int ncols, double alpha, const double* M, int64_t ld, const double* x, double beta,
              double* y) {
-    if (m <= 0 || ncols <= 0) return GPK_OK;
+    const int ny = trans ? ncols : m;
+    if (ny <= 0) return GPK_OK;
+    if ((trans ? m : ncols) <= 0) {   // empty product: y = beta * y (y = 0 for beta == 0, whatever y held)
+        gemv_n_finish<<<(ny + 255) / 256, 256, 0, h->stream>>>(ny, 0, alpha, nullptr, beta, y);
+        GPK_LAUNCH_CHECK(h);
+        return GPK_OK;
+    }
     if (!trans) {
         const int rblocks = (m + 127) / 128;
         int nch = (4 * 148 + rblocks - 1) / rblocks;               // ~4 CTAs per SM in total

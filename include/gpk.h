@@ -62,6 +62,19 @@ int gpk_debug_base_timing(gpk_handle h, long long* stamps_host);
  * one unstamped launch of the default kernel, [321..576] barrier arrival of four other warps per site, [577..896] phases of
  * tile warp 0 (the last two groups for chain >= 10 only). */
 int gpk_debug_ep_site_timing(gpk_handle h, int chain, long long* stamps_host);
+/* Development aid, not part of the drop-in surface (tests/test_gpu_gemm.py): issues exactly one internal DMMA GEMM with the
+ * descriptor given field by field and returns its status (GPK_EINVAL, without a launch, for R or S not a multiple of 64, K not
+ * a multiple of 16, an odd leading dimension or a pointer that is not 16-byte aligned).  Device pointers; for every 64 x 64
+ * tile selected by GPK_GEMM_TRI_OUT and each batch entry b (operands at base + b*stride):
+ *   D(r,s) = alpha * sum_{k in [kbeg,kend)} P(r,k) Q(s,k) + beta * Cin(r,s),  D(r,s) at D[s + r*ldd]
+ *   P(r,k) at P[k + r*ldp] if p_kcontig else P[r + k*ldp];  Q(s,k) likewise with q_kcontig
+ *   kbeg = max(KB_R ? r0 : 0, KB_S ? s0 : 0),  kend = min(K, KE_R ? r0 + 64 : K, KE_S ? s0 + 64 : K)
+ * with (r0, s0) the tile's first row / column.  TRI_OUT: only tiles with s0 >= r0; HEAVY_LAST: tiles in reverse launch
+ * order.  Cin may be NULL (no beta term) or equal to D. */
+enum { GPK_GEMM_TRI_OUT = 1, GPK_GEMM_KB_R = 2, GPK_GEMM_KB_S = 4, GPK_GEMM_KE_R = 8, GPK_GEMM_KE_S = 16, GPK_GEMM_HEAVY_LAST = 32 };
+int gpk_debug_gemm(gpk_handle h, const double* P, int64_t ldp, int64_t strideP, const double* Q, int64_t ldq, int64_t strideQ,
+                   double* D, int64_t ldd, int64_t strideD, const double* Cin, int64_t ldc, int64_t strideC, int R, int S, int K,
+                   int batch, double alpha, double beta, int p_kcontig, int q_kcontig, int flags);
 /* Launch sequences that callers repeat verbatim are captured into CUDA graphs and replayed: the single-problem
  * gpk_gp_nll_grad[_dev] evaluation (an optimiser's objective, GpPredictor.scala:126-142; same buffers and shape, new
  * hyper-parameters through device memory) from its second call on, the device-resident factor-only Cholesky up to n = 4096
