@@ -11,8 +11,10 @@
 
 #define GPK_TILE 128
 #define GPK_NPIPE 3
-#define GPK_NSIDE 16     // side streams (one per recursion depth, cyclic; batch group g starts at 4*g)
-#define GPK_NGROUP 4     // batch groups of the batched factorisation: group 0 on the handle's stream, the others on grp[]
+#define GPK_NSIDE 16     // side streams (one per recursion depth, cyclic; the second batch group starts at 4; the last one is
+                         // also the panel stream of the factor-only look-ahead driver)
+#define GPK_NGROUP 4     // grp[] has GPK_NGROUP - 1 main-priority streams: grp[0] runs the second batch group of the batched
+                         // factorisation, grp[0..2] the narrow flushes of the EP sweep
 #define GPK_NEVENTS 256  // fork/join event pool (cyclic)  // every internal matrix dimension / leading dimension is a multiple of this
 
 struct gpk_handle_s {
@@ -48,6 +50,13 @@ struct gpk_handle_s {
     int kernel_family;            // gpk_kernel_family: how (D, theta) arguments are interpreted
     char err[512];
 };
+// fork / join helpers of the multi-stream schedules
+struct StreamSwap {  // run the enclosed launches on another stream of the same handle
+    gpk_handle h; cudaStream_t saved;
+    StreamSwap(gpk_handle h_, cudaStream_t s) : h(h_), saved(h_->stream) { h->stream = s; }
+    ~StreamSwap() { h->stream = saved; }
+};
+static inline cudaEvent_t next_event(gpk_handle h) { return h->evpool[h->ev_next++ % GPK_NEVENTS]; }
 // ---- graph replay (gpk_graph.cu) ----
 #define GPK_NSLOTS 3
 enum { GPK_SLOT_EVAL = 0, GPK_SLOT_EP_SWEEP = 1, GPK_SLOT_POTRF = 2 };
@@ -230,17 +239,13 @@ int gpk_base_potrf_trtri(gpk_handle h, double* A, int64_t lda, double* Li, int64
                          int batch, int64_t strideA, int64_t strideLi, int info_stride, int coloff_stride);
 size_t gpk_chol_scratch_doubles(int N);
 int gpk_potrf_inv(gpk_handle h, double* A, double* Li, double* T, int N, int keep_L, int* info_dev, int batch = 1);
-// same, with a per-batch-group continuation: post(b0, cnt) is enqueued on the group's stream right behind its factorisation
-int gpk_potrf_inv_grouped(gpk_handle h, double* A, double* Li, double* T, int N, int keep_L, int* info_dev, int batch,
-                          const std::function<int(int, int)>& post);
 // Look-ahead driver for one large problem (see gpk_chol.cu): same results as gpk_potrf_inv; when Kinv != nullptr it also
 // accumulates K^-1 = Li^t Li (lower tiles) into Kinv (N x N, ld N, a buffer distinct from A and Li).
 bool gpk_use_pipelined(int N, int batch);
 // kinv_done != nullptr: returns without waiting for the K^-1 accumulation; the caller must cudaStreamWaitEvent(*kinv_done)
 // (when non-null) on its stream before reading Kinv.
 int gpk_potrf_inv_pipelined(gpk_handle h, double* A, double* Li, double* Kinv, double* T, int N, int keep_L, int* info_dev,
-                            cudaEvent_t* kinv_done = nullptr, int factor_only = 0, double* rhsB = nullptr, double* rhsV = nullptr,
-                            int rhsM = 0);
+                            cudaEvent_t* kinv_done = nullptr);
 // A -> L in place and V = L^-1 B (B, V: N x M, ld N; B destroyed); Li: N x N staging (holds L^-1 only when N is small)
 // on_rows (optional): called on the host, in order, once per block row of V -- rows [row0, row0 + rows) are final when `ready` fires
 // (the event is recorded on one of the handle's internal streams); lets a consumer of V start before the factorisation is done.
