@@ -520,11 +520,7 @@ int gpk_potrf_factor_solve(gpk_handle h, double* A, double* Li, double* T, int N
         return potrf_factor_pipelined(h, A, Li, T, N, info_dev, B, V, M, on_rows);
     int rc = gpk_potrf_inv(h, A, Li, T, N, 1, info_dev, 1);
     if (rc) return rc;
-    GemmDesc g = gemm_desc();                                       // V = L^-1 B: C(m,c) = sum_{k<=m} Li(m,k) B(k,c)
-    g.P = B; g.ldp = N; g.p_kcontig = 1;
-    g.Q = Li; g.ldq = N; g.q_kcontig = 0;
-    g.D = V; g.ldd = N; g.R = M; g.S = N; g.K = N; g.ke_s = 1; g.heavy_last = 1;
-    rc = gpk_gemm(h, g);
+    rc = gpk_trmm_lower(h, Li, N, B, V, M);
     if (rc || !on_rows) return rc;
     cudaEvent_t evV = next_event(h);                                // all rows at once
     GPK_CUDA(h, cudaEventRecord(evV, h->stream));
@@ -584,5 +580,16 @@ int gpk_lauum_lower(gpk_handle h, const double* Li, double* Kinv, int N, int bat
     g.D = Kinv; g.ldd = N;
     g.R = N; g.S = N; g.K = N; g.kb_r = 1; g.kb_s = 1; g.tri_out = 1;
     g.batch = batch; g.strideP = g.strideQ = g.strideD = (int64_t)N * N;
+    return gpk_gemm(h, g);
+}
+
+int gpk_trmm_lower(gpk_handle h, const double* Li, int N, const double* B, double* V, int M, int batch) {
+    // V(m,c) = sum_{k <= m} Li(m,k) B(k,c)
+    GemmDesc g = gemm_desc();
+    g.P = B; g.ldp = N; g.p_kcontig = 1;   // P(r,k) = B(k,r)
+    g.Q = Li; g.ldq = N; g.q_kcontig = 0;  // Q(s,k) = Li(s,k)
+    g.D = V; g.ldd = N;
+    g.R = M; g.S = N; g.K = N; g.ke_s = 1; g.heavy_last = 1;
+    g.batch = batch; g.strideP = g.strideD = (int64_t)N * M; g.strideQ = (int64_t)N * N;
     return gpk_gemm(h, g);
 }

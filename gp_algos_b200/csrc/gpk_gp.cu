@@ -207,7 +207,7 @@ __global__ void __launch_bounds__(256) ucb_grad_kernel(const double* __restrict_
         __syncthreads();
     }
     if (threadIdx.x == 0) {
-        const double sigma = (cp.sf2 + cp.sn2) - colsq[c];       // k(x,x) incl. the i==j noise term (MatrixUtils.scala:63) - v^t v
+        const double sigma = gpk_prior_var(cp) - colsq[c];       // k(x,x) - v^t v
         const double coeff = kparam / (2 * sqrt(sigma));
         grad[c + (int64_t)d * ms] = sa[0] + (0.0 - 2.0 * sb[0]) * coeff;
         if (d == 0) { ucb[c] = mean[c] + kparam * sqrt(sigma); var[c] = sigma; }
@@ -263,6 +263,20 @@ __global__ void __launch_bounds__(256) model_grow_kernel(const double* __restric
 }
 
 }  // namespace
+
+int gpk_posterior(gpk_handle h, const double* dX, int n, int64_t ldx, const double* dXs, int ms, const double* Li,
+                  const double* alpha, int N, const CovParams& cp, double* KsT, double* mean, double* V, int nv, double* vsq,
+                  int batch, int64_t strideX, int64_t strideXs, const ProblemParams* pp_dev) {
+    const int M = gpk_pad(ms);
+    const int64_t sK = (int64_t)N * M;
+    int rc = gpk_cov_cross(h, dX, n, ldx, dXs, ms, ms, cp, KsT, N, N, M, batch, strideX, strideXs, sK, pp_dev);  // GpPredictor.scala:53
+    if (rc) return rc;
+    rc = gpk_colwise_dot(h, KsT, N, N, ms, alpha, mean, 0, batch, sK, N, M);                                       // :54
+    if (rc || !V) return rc;
+    rc = gpk_trmm_lower(h, Li, N, KsT, V, gpk_pad(nv), batch);                                                     // :55
+    if (rc || !vsq) return rc;
+    return gpk_colwise_dot(h, V, N, N, nv, nullptr, vsq, 1, batch, sK, 0, M);                                      // :56, diagonal
+}
 
 extern "C" {
 
@@ -533,8 +547,8 @@ int gpk_gp_model_append(gpk_handle h, gpk_model m, const double* x_new, double y
     if (rc) return rc;
     rc = gpk_trmv_lower_t(h, m->Li, N, dl, dw);                                         // w = L^-t l
     if (rc) return rc;
-    // k(x,x) with the i == j noise term (MatrixUtils.scala:63) and the Option sigmaNoise of the fit (GpPredictor.scala:116-117)
-    const double kss = m->pp.cp.sf2 + m->pp.cp.sn2 + (has_s ? s : 0.0);
+    // k(x,x) and the Option sigmaNoise of the fit (GpPredictor.scala:116-117)
+    const double kss = gpk_prior_var(m->pp.cp) + (has_s ? s : 0.0);
     model_append_kernel<<<(n + 256) / 256, 256, 0, h->stream>>>(m->Li, N, n, m->alpha, m->X, m->ldx, D, dx, dw, ddots, kss, y_new,
                                                                 h->d_info, dres);
     GPK_LAUNCH_CHECK(h);
@@ -573,22 +587,11 @@ int gpk_gp_model_predict(gpk_handle h, gpk_model m, const double* Xs, int ms, in
     double* dVar = dMean + M;
     int rc = gpk_upload_matrix(h, dXs, Xs, ms, D, ldxs);
     if (rc) return rc;
-    // K*^t = k(X, X*) : N x M with zero padding (GpPredictor.scala:53, no noise)
-    rc = gpk_cov_cross(h, m->X, n, m->ldx, dXs, ms, ms, cp, dKsT, N, N, M);
+    // V is skipped when only the mean is wanted (the GP-UKF transition / observation functions, GPUnscentedKalmanFilter.scala:77-90,
+    // read nothing else); the full covariance needs no column sums
+    rc = gpk_posterior(h, m->X, n, m->ldx, dXs, ms, m->Li, m->alpha, N, cp, dKsT, dMean, (sigma || V) ? dV : nullptr, ms,
+                       (sigma && !want_full_cov) ? dVar : nullptr);
     if (rc) return rc;
-    // mean = K* alpha (GpPredictor.scala:54)
-    rc = gpk_colwise_dot(h, dKsT, N, N, ms, m->alpha, dMean, 0);
-    if (rc) return rc;
-    // V = L^-1 K*^t (GpPredictor.scala:55): C(i,c) = sum_{k<=i} Li(i,k) KsT(k,c).  Skipped when only the mean is wanted
-    // (the GP-UKF transition / observation functions, GPUnscentedKalmanFilter.scala:77-90, read nothing else).
-    GemmDesc g = gemm_desc();
-    if (sigma || V) {
-        g.P = dKsT; g.ldp = N; g.p_kcontig = 1;
-        g.Q = m->Li; g.ldq = N; g.q_kcontig = 0;
-        g.D = dV; g.ldd = N; g.R = M; g.S = N; g.K = N; g.ke_s = 1; g.heavy_last = 1;
-        rc = gpk_gemm(h, g);
-        if (rc) return rc;
-    }
     if (mean) GPK_CUDA(h, cudaMemcpyAsync(mean, dMean, (size_t)ms * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
     if (sigma) {
         if (want_full_cov) {
@@ -596,7 +599,7 @@ int gpk_gp_model_predict(gpk_handle h, gpk_model m, const double* Xs, int ms, in
             GPK_CUDA(h, cudaMemsetAsync(dSig, 0, (size_t)M * M * sizeof(double), h->stream));
             rc = gpk_cov_sym_full(h, dXs, ms, ms, cp, dSig, M);
             if (rc) return rc;
-            g = gemm_desc();
+            GemmDesc g = gemm_desc();
             g.P = dV; g.ldp = N; g.p_kcontig = 1;
             g.Q = dV; g.ldq = N; g.q_kcontig = 1;
             g.D = dSig; g.ldd = M; g.Cin = dSig; g.ldc = M; g.R = M; g.S = M; g.K = N; g.alpha = -1.0; g.beta = 1.0;
@@ -605,8 +608,6 @@ int gpk_gp_model_predict(gpk_handle h, gpk_model m, const double* Xs, int ms, in
             GPK_CUDA(h, cudaMemcpy2DAsync(sigma, (size_t)lds * sizeof(double), dSig, (size_t)M * sizeof(double),
                                           (size_t)ms * sizeof(double), (size_t)ms, cudaMemcpyDeviceToHost, h->stream));
         } else {
-            rc = gpk_colwise_dot(h, dV, N, N, ms, nullptr, dVar, 1);
-            if (rc) return rc;
             GPK_CUDA(h, cudaMemcpyAsync(sigma, dVar, (size_t)ms * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
         }
     }
@@ -614,10 +615,8 @@ int gpk_gp_model_predict(gpk_handle h, gpk_model m, const double* Xs, int ms, in
                                          (size_t)ms, cudaMemcpyDeviceToHost, h->stream));
     rc = gpk_synchronize(h);
     if (rc) return rc;
-    if (sigma && !want_full_cov) {
-        const double kss = cp.sf2 + cp.sn2;  // k(x*,x*) incl. the i==j noise term
-        for (int i = 0; i < ms; ++i) sigma[i] = kss - sigma[i];
-    }
+    if (sigma && !want_full_cov)
+        for (int i = 0; i < ms; ++i) sigma[i] = gpk_prior_var(cp) - sigma[i];
     return GPK_OK;
 }
 
@@ -646,19 +645,9 @@ int gpk_gp_model_ucb(gpk_handle h, gpk_model m, const double* Xs, int ms, int64_
     double* dGrad = dVar + M;
     int rc = gpk_upload_matrix(h, dXs, Xs, ms, D, ldxs);
     if (rc) return rc;
-    rc = gpk_cov_cross(h, m->X, n, m->ldx, dXs, ms, ms, cp, dKsT, N, N, M);     // k* (GpPredictor.scala:53)
+    rc = gpk_posterior(h, m->X, n, m->ldx, dXs, ms, m->Li, m->alpha, N, cp, dKsT, dMean, dV, ms, dSq);
     if (rc) return rc;
-    rc = gpk_colwise_dot(h, dKsT, N, N, ms, m->alpha, dMean, 0);                 // mean (GpPredictor.scala:54)
-    if (rc) return rc;
-    GemmDesc g = gemm_desc();                                                    // V = L^-1 K*^t (GpPredictor.scala:55)
-    g.P = dKsT; g.ldp = N; g.p_kcontig = 1;
-    g.Q = m->Li; g.ldq = N; g.q_kcontig = 0;
-    g.D = dV; g.ldd = N; g.R = M; g.S = N; g.K = N; g.ke_s = 1; g.heavy_last = 1;
-    rc = gpk_gemm(h, g);
-    if (rc) return rc;
-    rc = gpk_colwise_dot(h, dV, N, N, ms, nullptr, dSq, 1);                      // v^t v
-    if (rc) return rc;
-    g = gemm_desc();                                                             // U = L^-t V: U(i,c) = sum_{k>=i} Li(k,i) V(k,c)
+    GemmDesc g = gemm_desc();                                                    // U = L^-t V: U(i,c) = sum_{k>=i} Li(k,i) V(k,c)
     g.P = dV; g.ldp = N; g.p_kcontig = 1;
     g.Q = m->Li; g.ldq = N; g.q_kcontig = 1;
     g.D = dU; g.ldd = N; g.R = M; g.S = N; g.K = N; g.kb_s = 1;
@@ -679,31 +668,49 @@ int gpk_gp_model_ucb(gpk_handle h, gpk_model m, const double* Xs, int ms, int64_
 // (GPUnscentedKalmanFilter.scala:77-90: one GP per state / observation dimension, each asked for its mean at every sigma
 // point).  mean[j*ms + i] = mean of model j at row i.  Models may differ in training set, targets and hyper-parameters.
 int gpk_gp_models_mean(gpk_handle h, const gpk_model* models, int nmodels, const double* Xs, int ms, int64_t ldxs, double* mean) {
+    return gpk_gp_models_mean_var(h, models, nmodels, Xs, ms, ldxs, mean, nullptr);
+}
+
+// GPUnscentedKalmanFilter.scala:77-90 + :138-147 in one call: means AND variances (diagonal of computePosterior's sigma,
+// including noiseVar^2, MatrixUtils.scala:63) of nmodels resident models at the same ms test rows.
+int gpk_gp_models_mean_var(gpk_handle h, const gpk_model* models, int nmodels, const double* Xs, int ms, int64_t ldxs,
+                           double* mean, double* var) {
     if (!h || !models || nmodels <= 0 || !Xs || ms <= 0 || ldxs < ms || !mean)
-        return gpk_set_error(h, GPK_EINVAL, "gpk_gp_models_mean: bad arguments");
+        return gpk_set_error(h, GPK_EINVAL, "gpk_gp_models_mean_var: bad arguments");
     GPK_CUDA(h, cudaSetDevice(h->device));
     const int D = models[0]->D, M = gpk_pad(ms);
     int Nmax = 0;
     for (int j = 0; j < nmodels; ++j) {
-        if (!models[j] || models[j]->D != D) return gpk_set_error(h, GPK_EINVAL, "gpk_gp_models_mean: models disagree on D");
+        if (!models[j] || models[j]->D != D) return gpk_set_error(h, GPK_EINVAL, "gpk_gp_models_mean_var: models disagree on D");
         if (models[j]->N > Nmax) Nmax = models[j]->N;
     }
     ARENA_OR_FAIL(dXs, double*, h, ARENA_X, (size_t)ms * D * sizeof(double));
-    ARENA_OR_FAIL(buf, double*, h, ARENA_IO2, ((size_t)Nmax * M + (size_t)nmodels * M) * sizeof(double));
+    // KsT (Nmax x M), mean (nmodels x M); with var also V (Nmax x M), vsq (nmodels x M)
+    const size_t nKm = (size_t)Nmax * M + (size_t)nmodels * M;
+    ARENA_OR_FAIL(buf, double*, h, ARENA_IO2, (var ? 2 : 1) * nKm * sizeof(double));
     double* dKsT = buf;
-    double* dMean = buf + (size_t)Nmax * M;
+    double* dMean = dKsT + (size_t)Nmax * M;
+    double* dV = var ? buf + nKm : nullptr;
+    double* dVsq = var ? dV + (size_t)Nmax * M : nullptr;
     int rc = gpk_upload_matrix(h, dXs, Xs, ms, D, ldxs);
     if (rc) return rc;
     for (int j = 0; j < nmodels; ++j) {
         gpk_model m = models[j];
-        rc = gpk_cov_cross(h, m->X, m->n, m->ldx, dXs, ms, ms, m->pp.cp, dKsT, m->N, m->N, M);   // GpPredictor.scala:53
-        if (rc) return rc;
-        rc = gpk_colwise_dot(h, dKsT, m->N, m->N, ms, m->alpha, dMean + (size_t)j * M, 0);         // :54
+        rc = gpk_posterior(h, m->X, m->n, m->ldx, dXs, ms, m->Li, m->alpha, m->N, m->pp.cp, dKsT, dMean + (size_t)j * M, dV, ms,
+                           var ? dVsq + (size_t)j * M : nullptr);
         if (rc) return rc;
     }
     GPK_CUDA(h, cudaMemcpy2DAsync(mean, (size_t)ms * sizeof(double), dMean, (size_t)M * sizeof(double), (size_t)ms * sizeof(double),
                                   (size_t)nmodels, cudaMemcpyDeviceToHost, h->stream));
-    return gpk_synchronize(h);
+    if (var)
+        GPK_CUDA(h, cudaMemcpy2DAsync(var, (size_t)ms * sizeof(double), dVsq, (size_t)M * sizeof(double), (size_t)ms * sizeof(double),
+                                      (size_t)nmodels, cudaMemcpyDeviceToHost, h->stream));
+    rc = gpk_synchronize(h);
+    if (rc) return rc;
+    if (var)
+        for (int j = 0; j < nmodels; ++j)
+            for (int i = 0; i < ms; ++i) var[(size_t)j * ms + i] = gpk_prior_var(models[j]->pp.cp) - var[(size_t)j * ms + i];
+    return GPK_OK;
 }
 
 int gpk_gp_predict(gpk_handle h, const double* X, int n, int D, int64_t ldx, const double* y, const double* Xs, int ms,
@@ -759,19 +766,8 @@ int gpk_gp_predict_batched(gpk_handle h, int B, const double* X, int n, int D, i
         rc = fit_core(h, w, bc, dX, n, D, n, sX, dy, pp0, 0, w.Li, w.alpha, dll, 1, w.info_dev);
         if (rc) break;
         // predictions use the kernel without the Option sigmaNoise: extra_diag does not enter cross-covariances
-        const ProblemParams* ppd = bc > 1 ? w.pp_dev : nullptr;
-        rc = gpk_cov_cross(h, dX, n, n, dXs, ms, ms, pp0.cp, dKsT, N, N, M, bc, sX, sXs, (int64_t)N * M, ppd);
-        if (rc) break;
-        rc = gpk_colwise_dot(h, dKsT, N, N, ms, w.alpha, dMean, 0, bc, (int64_t)N * M, N, M);
-        if (rc) break;
-        GemmDesc g = gemm_desc();
-        g.P = dKsT; g.ldp = N; g.p_kcontig = 1; g.strideP = (int64_t)N * M;
-        g.Q = w.Li; g.ldq = N; g.q_kcontig = 0; g.strideQ = (int64_t)N * N;
-        g.D = dV; g.ldd = N; g.strideD = (int64_t)N * M; g.batch = bc;
-        g.R = M; g.S = N; g.K = N; g.ke_s = 1; g.heavy_last = 1;
-        rc = gpk_gemm(h, g);
-        if (rc) break;
-        rc = gpk_colwise_dot(h, dV, N, N, ms, nullptr, dVar, 1, bc, (int64_t)N * M, 0, M);
+        rc = gpk_posterior(h, dX, n, n, dXs, ms, w.Li, w.alpha, N, pp0.cp, dKsT, dMean, dV, ms, dVar, bc, sX, sXs,
+                           bc > 1 ? w.pp_dev : nullptr);
         if (rc) break;
         cudaError_t e = cudaMemcpy2DAsync(mean + (size_t)b0 * ms, (size_t)ms * sizeof(double), dMean, (size_t)M * sizeof(double),
                                           (size_t)ms * sizeof(double), (size_t)bc, cudaMemcpyDeviceToHost, h->stream);
@@ -781,12 +777,9 @@ int gpk_gp_predict_batched(gpk_handle h, int B, const double* X, int n, int D, i
         if (e == cudaSuccess) e = cudaMemcpyAsync(hinfo + b0, w.info_dev, (size_t)bc * sizeof(int), cudaMemcpyDeviceToHost, h->stream);
         if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
         if (e != cudaSuccess) { rc = gpk_set_error(h, GPK_ECUDA, "batched predict: %s", cudaGetErrorString(e)); break; }
+        const ProblemParams* hp = (const ProblemParams*)h->pp_host;   // the chunk's records, as stage_params built them
         for (int b = 0; b < bc; ++b) {
-            const double* th = thetas + (size_t)(b0 + b) * gpk_theta_len(h, D);
-            CovParams cpb;
-            gpk_make_cov_params(h, th, D, 0, 0.0, &cpb);
-            const double kss = cpb.sf2 + cpb.sn2;  // k(x*,x*) incl. the i==j noise term (MatrixUtils.scala:63)
-            for (int i = 0; i < ms; ++i) var[(size_t)(b0 + b) * ms + i] = kss - var[(size_t)(b0 + b) * ms + i];
+            for (int i = 0; i < ms; ++i) var[(size_t)(b0 + b) * ms + i] = gpk_prior_var(hp[b].cp) - var[(size_t)(b0 + b) * ms + i];
             if (info) info[b0 + b] = hinfo[b0 + b];
             if (hinfo[b0 + b] && !bad) { bad = 1; h->last_info = hinfo[b0 + b]; }
         }

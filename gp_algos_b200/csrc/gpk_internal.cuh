@@ -150,6 +150,8 @@ struct CovParams {
     double extra_diag;   // Option sigmaNoise (un-squared), 0 when None
     double inv_ls2[GPK_MAX_D];  // SE-ARD: 1/(ls*ls).             Co2: hp1..hp11, then pow(hp2,-3), pow(hp4,-3), pow(hp5,-3), pow(hp7,-3), pow(hp10,-3)
 };
+// k(x, x) with the i == j noise term (MatrixUtils.scala:63): the prior variance a posterior variance is taken from
+static inline __host__ __device__ double gpk_prior_var(const CovParams& cp) { return cp.sf2 + cp.sn2; }
 static inline int gpk_theta_len(const gpk_handle_s* h, int D) { return h->kernel_family == GPK_KERNEL_CO2 ? GPK_CO2_NPARAMS : D + 2; }
 
 #ifdef __CUDACC__
@@ -211,6 +213,18 @@ struct gpk_model_s {
     double s;       // ... replayed by gpk_gp_model_append
 };
 
+// computePosterior (GpPredictor.scala:45-58) up to the prior variance, for `batch` GPs of padded size N at ms test rows
+// (gpk_gp.cu).  Problem b: X at dX + b*strideX (n rows, ld ldx), X* at dXs + b*strideXs (ld ms), Li (N x N) at + b*N*N,
+// alpha (N) at + b*N, hyper-parameters cp (batch == 1) or pp_dev[b].  With M = gpk_pad(ms) it writes, at + b*N*M resp. + b*M:
+//   KsT   N x M (ld N)   k(X, X*) with zero padding
+//   mean  M              K* alpha
+//   V     N x M (ld N)   Li KsT over the first gpk_pad(nv) columns only, so with batch == 1 N x gpk_pad(nv) suffices
+//                        (nv <= ms; nv == ms when batch > 1); skipped when null
+//   vsq   M              column sums of squares of V over the first nv columns; needs V; skipped when null
+int gpk_posterior(gpk_handle h, const double* dX, int n, int64_t ldx, const double* dXs, int ms, const double* Li,
+                  const double* alpha, int N, const CovParams& cp, double* KsT, double* mean, double* V, int nv, double* vsq,
+                  int batch = 1, int64_t strideX = 0, int64_t strideXs = 0, const ProblemParams* pp_dev = nullptr);
+
 // ---------------------------------------------------------------------------------------------
 // covariance (gpk_cov.cu)
 // ---------------------------------------------------------------------------------------------
@@ -262,6 +276,10 @@ int gpk_trsm_padded(gpk_handle h, const double* Lw, double* Di, int N, int backw
 int gpk_trtri_lower(gpk_handle h, const double* L, double* Li, double* T, int N);
 // Kinv (lower triangle incl. diagonal tiles in full) = Li^t Li
 int gpk_lauum_lower(gpk_handle h, const double* Li, double* Kinv, int N, int batch = 1);
+// V = Li B for `batch` problems: B, V are N x M (ld N, M a multiple of 64) at + b*N*M, Li at + b*N*N.  Li is read up to the
+// diagonal 64-tile of each row tile only (zero above the diagonal inside it, as gpk_potrf_inv leaves it); the blocks above
+// may hold anything -- a resident model's are uninitialised memory.
+int gpk_trmm_lower(gpk_handle h, const double* Li, int N, const double* B, double* V, int M, int batch = 1);
 
 // ---------------------------------------------------------------------------------------------
 // vectors / reductions / gradient (gpk_vec.cu, gpk_grad.cu)

@@ -217,72 +217,9 @@ __global__ void ukf_init(UkfDims dm, UkfState st, const double* init_mean, const
     if (b == 0) st.info[0] = 0;
 }
 
-// posterior means of `nm` resident models at the ms rows of dXs (ld ms) -> dMean[j * Mp + r]; nvar > 0: |L^-1 k*|^2 of the first
-// nvar rows -> dVsq[j * Vp + r] (Vp = pad128(nvar)).  KsT: Nmax x Mp scratch, V: Nmax x Vp scratch.
-int models_eval(gpk_handle h, const gpk_model* models, int nm, const double* dXs, int ms, int Mp, double* dKsT, double* dMean,
-                int nvar, int Vp, double* dV, double* dVsq) {
-    for (int j = 0; j < nm; ++j) {
-        gpk_model m = models[j];
-        int rc = gpk_cov_cross(h, m->X, m->n, m->ldx, dXs, ms, ms, m->pp.cp, dKsT, m->N, m->N, Mp);     // GpPredictor.scala:53
-        if (rc) return rc;
-        rc = gpk_colwise_dot(h, dKsT, m->N, m->N, ms, m->alpha, dMean + (size_t)j * Mp, 0);               // :54
-        if (rc) return rc;
-        if (nvar > 0) {
-            GemmDesc g = gemm_desc();                                                                     // V = L^-1 K*^t (:55)
-            g.P = dKsT; g.ldp = m->N; g.p_kcontig = 1;
-            g.Q = m->Li; g.ldq = m->N; g.q_kcontig = 0;
-            g.D = dV; g.ldd = m->N; g.R = Vp; g.S = m->N; g.K = m->N; g.ke_s = 1; g.heavy_last = 1;
-            rc = gpk_gemm(h, g);
-            if (rc) return rc;
-            rc = gpk_colwise_dot(h, dV, m->N, m->N, nvar, nullptr, dVsq + (size_t)j * Vp, 1);
-            if (rc) return rc;
-        }
-    }
-    return GPK_OK;
-}
-
 }  // namespace
 
 extern "C" {
-
-// GPUnscentedKalmanFilter.scala:77-90 + :138-147 in one call: means AND variances (diagonal of computePosterior's sigma,
-// including noiseVar^2, MatrixUtils.scala:63) of nmodels resident models at the same ms test rows.
-int gpk_gp_models_mean_var(gpk_handle h, const gpk_model* models, int nmodels, const double* Xs, int ms, int64_t ldxs,
-                           double* mean, double* var) {
-    if (!h || !models || nmodels <= 0 || !Xs || ms <= 0 || ldxs < ms || !mean)
-        return gpk_set_error(h, GPK_EINVAL, "gpk_gp_models_mean_var: bad arguments");
-    GPK_CUDA(h, cudaSetDevice(h->device));
-    const int D = models[0]->D, M = gpk_pad(ms);
-    int Nmax = 0;
-    for (int j = 0; j < nmodels; ++j) {
-        if (!models[j] || models[j]->D != D) return gpk_set_error(h, GPK_EINVAL, "gpk_gp_models_mean_var: models disagree on D");
-        if (models[j]->N > Nmax) Nmax = models[j]->N;
-    }
-    double* dXs = (double*)gpk_arena(h, ARENA_X, (size_t)ms * D * sizeof(double));
-    double* buf = (double*)gpk_arena(h, ARENA_IO2, ((size_t)2 * Nmax * M + (size_t)2 * nmodels * M) * sizeof(double));
-    if (!dXs || !buf) return GPK_ENOMEM;
-    double* dKsT = buf;
-    double* dV = dKsT + (size_t)Nmax * M;
-    double* dMean = dV + (size_t)Nmax * M;
-    double* dVsq = dMean + (size_t)nmodels * M;
-    int rc = gpk_upload_matrix(h, dXs, Xs, ms, D, ldxs);
-    if (rc) return rc;
-    rc = models_eval(h, models, nmodels, dXs, ms, M, dKsT, dMean, var ? ms : 0, M, dV, dVsq);
-    if (rc) return rc;
-    GPK_CUDA(h, cudaMemcpy2DAsync(mean, (size_t)ms * sizeof(double), dMean, (size_t)M * sizeof(double), (size_t)ms * sizeof(double),
-                                  (size_t)nmodels, cudaMemcpyDeviceToHost, h->stream));
-    if (var)
-        GPK_CUDA(h, cudaMemcpy2DAsync(var, (size_t)ms * sizeof(double), dVsq, (size_t)M * sizeof(double), (size_t)ms * sizeof(double),
-                                      (size_t)nmodels, cudaMemcpyDeviceToHost, h->stream));
-    rc = gpk_synchronize(h);
-    if (rc) return rc;
-    if (var)
-        for (int j = 0; j < nmodels; ++j) {
-            const double kss = models[j]->pp.cp.sf2 + models[j]->pp.cp.sn2;     // k(x*,x*) incl. the i == j noise term
-            for (int i = 0; i < ms; ++i) var[(size_t)j * ms + i] = kss - var[(size_t)j * ms + i];
-        }
-    return GPK_OK;
-}
 
 int gpk_gpukf_filter(gpk_handle h, const gpk_model* sys_models, int d, const gpk_model* obs_models, int p, int B, int T,
                      const double* y, const double* init_mean, const double* init_cov, double alpha, double beta, double kappa,
@@ -323,7 +260,7 @@ int gpk_gpukf_filter(gpk_handle h, const gpk_model* sys_models, int d, const gpk
     GPK_CUDA(h, cudaMemcpyAsync(dC0, init_cov, (size_t)B * d * d * sizeof(double), cudaMemcpyHostToDevice, h->stream));
     for (int j = 0; j < d + p; ++j) {
         gpk_model m = j < d ? sys_models[j] : obs_models[j - d];
-        h->h_pinned[128 + j] = m->pp.cp.sf2 + m->pp.cp.sn2;       // k(x,x) with the i == j noise term (MatrixUtils.scala:63)
+        h->h_pinned[128 + j] = gpk_prior_var(m->pp.cp);
     }
     GPK_CUDA(h, cudaMemcpyAsync(kss, h->h_pinned + 128, (size_t)(d + p) * sizeof(double), cudaMemcpyHostToDevice, h->stream));
     // weights (UnscentedKalmanFilter.scala:87,96-97)
@@ -336,12 +273,21 @@ int gpk_gpukf_filter(gpk_handle h, const gpk_model* sys_models, int d, const gpk
     for (int t = 1; t < T; ++t) {
         ukf_sigma1<<<nb, 64, 0, h->stream>>>(dm, st, c, t, SP);
         GPK_LAUNCH_CHECK(h);
-        int rc = models_eval(h, sys_models, d, SP, dm.M, dm.Mp, KsT, gmean, B, dm.Bp, V, vsq);
-        if (rc) return rc;
+        // means at every sigma point, |L^-1 k*|^2 at the B central ones (rows 0 .. B-1)
+        for (int j = 0; j < d; ++j) {
+            const gpk_model m = sys_models[j];
+            int rc = gpk_posterior(h, m->X, m->n, m->ldx, SP, dm.M, m->Li, m->alpha, m->N, m->pp.cp, KsT, gmean + (size_t)j * dm.Mp, V,
+                                   B, vsq + (size_t)j * dm.Bp);
+            if (rc) return rc;
+        }
         ukf_predict<<<nb, 64, 0, h->stream>>>(dm, st, c, w0m, w0c, wic, t, SP, gmean, vsq, kss, SP2);
         GPK_LAUNCH_CHECK(h);
-        rc = models_eval(h, obs_models, p, SP2, dm.M, dm.Mp, KsT, gmean, B, dm.Bp, V, vsq);
-        if (rc) return rc;
+        for (int j = 0; j < p; ++j) {
+            const gpk_model m = obs_models[j];
+            int rc = gpk_posterior(h, m->X, m->n, m->ldx, SP2, dm.M, m->Li, m->alpha, m->N, m->pp.cp, KsT, gmean + (size_t)j * dm.Mp, V,
+                                   B, vsq + (size_t)j * dm.Bp);
+            if (rc) return rc;
+        }
         ukf_update<<<nb, 64, 0, h->stream>>>(dm, st, w0m, w0c, wic, t, gmean, vsq, kss + d, dY, compute_ll, dOutM, dOutC);
         GPK_LAUNCH_CHECK(h);
     }

@@ -1,5 +1,7 @@
 """GPU parity for the batched independent-GP entry points (BASELINE.json config 4) through the C ABI."""
 import os
+import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -9,6 +11,7 @@ from gp_algos_b200 import batched
 from oracle import gp_oracle as orc
 
 pytestmark = pytest.mark.gpu
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 G = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 RTOL = 1e-9
 
@@ -170,3 +173,41 @@ def test_full_batch_is_bit_reproducible_over_many_runs():
             first = res
         else:
             assert np.array_equal(res, first), f"run {rep} differs from run 0 in problems {np.unique(np.argwhere(res != first) // (D + 3))[:5]}"
+
+
+# GPK_BATCH_GB = 0.032 GiB holds 5 problems of n = 300 (N = 384, D = 4): about 5.95 MiB each (L, L^-1, the Cholesky scratch and
+# the vectors of make_work, csrc/gpk_gp.cu), so the 19 problems run in chunks of 5, 5, 5 and 4.  n stays far below 4096, where a
+# chunk of one problem would take the look-ahead driver.
+CHUNK_ENV = {"GPK_BATCH_GB": "0.032"}
+
+
+def _chunk_results(path):
+    """Runs in the child and in the parent: both batched entry points on 19 problems with their own X and X*."""
+    from gp_algos_b200 import _lib
+    B, n, D, m = 19, 300, 4, 9
+    rng = np.random.default_rng(31)
+    X = rng.uniform(0, 1, size=(B, n, D)); Xs = rng.uniform(0, 1, size=(B, m, D))
+    ys = np.stack([np.sin(X[b] @ rng.standard_normal(D)) + 0.1 * rng.standard_normal(n) for b in range(B)])
+    th = np.stack([orc.pack_theta(10 ** rng.uniform(-0.3, 0.3), 10 ** rng.uniform(-0.5, 0.2, size=D), 0.1) for _ in range(B)])
+    h = _lib.default_handle()
+    l0 = h.launch_count()
+    mean, var, ll, info = batched.predict_batched(X, ys, th, Xs)
+    launches = h.launch_count() - l0
+    ll_g, grad, info_g = batched.log_likelihood_with_derivatives_batched(X, ys, th)
+    np.savez(path, mean=mean, var=var, ll=ll, info=info, ll_g=ll_g, grad=grad, info_g=info_g, launches=launches)
+
+
+def test_chunked_batch_equals_one_chunk(tmp_path):
+    """A batch larger than GPK_BATCH_GB runs chunk by chunk.  The budget is read once per process, so the chunked run is a child.
+    Every problem is computed on its own, so the chunks must reproduce the one-chunk run bit for bit."""
+    code = ("import sys; sys.path.insert(0, sys.argv[1]); from tests.test_gpu_batched import _chunk_results; "
+            "_chunk_results(sys.argv[2])")
+    r = subprocess.run([sys.executable, "-c", code, ROOT, str(tmp_path / "chunked.npz")], env=dict(os.environ, **CHUNK_ENV),
+                       capture_output=True, text=True, timeout=600)
+    assert r.returncode == 0, f"child with {CHUNK_ENV} failed:\n{r.stderr[-4000:]}"
+    _chunk_results(tmp_path / "whole.npz")
+    got, want = np.load(tmp_path / "chunked.npz"), np.load(tmp_path / "whole.npz")
+    assert got["launches"] > want["launches"], "GPK_BATCH_GB did not split the batch"
+    assert np.all(want["info"] == 0) and np.all(want["info_g"] == 0)
+    for k in ("mean", "var", "ll", "info", "ll_g", "grad", "info_g"):
+        assert np.array_equal(got[k], want[k]), f"{k}: chunked run differs from the one-chunk run"
