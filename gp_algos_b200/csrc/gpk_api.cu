@@ -21,6 +21,17 @@ int gpk_set_error(gpk_handle h, int status, const char* fmt, ...) {
     return status;
 }
 
+int gpk_check_args(gpk_handle h, const char* fn, bool ok, int n, int n_min, int64_t ldx, int D, int nparams) {
+    const char* bad = !h ? "null handle"
+                    : (!ok || n < n_min || ldx < n) ? "bad arguments"
+                    : (D < 1 || D > GPK_MAX_D) ? "feature dimension out of range"
+                    : (nparams < 0 || nparams > gpk_theta_len(h, D)) ? "nparams out of range"
+                    : nullptr;
+    if (!bad) return GPK_OK;
+    return gpk_set_error(h, GPK_EINVAL, "%s: %s (n=%d, ldx=%lld, D=%d of 1..%d, nparams=%d)", fn, bad, n, (long long)ldx, D,
+                         GPK_MAX_D, nparams);
+}
+
 void* gpk_arena(gpk_handle h, int which, size_t bytes) {
     if (bytes <= h->arena_bytes[which] && h->arena[which]) return h->arena[which];
     if (h->cap) {  // stream capture in progress: allocation would synchronise; the capturing caller falls back to eager launches
@@ -62,6 +73,17 @@ int gpk_download_matrix(gpk_handle h, double* dst, int64_t ld, const double* src
     return GPK_OK;
 }
 
+int gpk_upload_padded(gpk_handle h, double* dst, int N, const double* src, int n, int64_t lds, int form, int* d_notsym) {
+    ARENA_OR_FAIL(dIn, double*, h, ARENA_IO, (size_t)n * n * sizeof(double));
+    int rc = gpk_upload_matrix(h, dIn, src, n, n, lds);
+    return rc ? rc : gpk_load_padded(h, dst, N, dIn, n, n, form, d_notsym);
+}
+int gpk_download_tri(gpk_handle h, double* dst, int64_t ldd, const double* src, int N, int n, int transpose) {
+    ARENA_OR_FAIL(dOut, double*, h, ARENA_IO, (size_t)n * n * sizeof(double));
+    int rc = gpk_store_tri(h, dOut, n, src, N, n, transpose);
+    return rc ? rc : gpk_download_matrix(h, dst, ldd, dOut, n, n);
+}
+
 // after a single factorisation: fetch info, map to status
 int gpk_finish_info(gpk_handle h) {
     int info = 0;
@@ -71,10 +93,6 @@ int gpk_finish_info(gpk_handle h) {
     if (info != 0) return gpk_set_error(h, GPK_ENOTPD, "matrix not positive definite: leading minor %d", info);
     return GPK_OK;
 }
-
-#define ARENA_OR_FAIL(ptr, type, h, which, bytes)           \
-    type ptr = (type)gpk_arena((h), (which), (bytes));      \
-    if (!ptr) return GPK_ENOMEM
 
 extern "C" {
 
@@ -184,20 +202,21 @@ int gpk_synchronize(gpk_handle h) {
 // covariance
 // ------------------------------------------------------------------------------------------------
 int gpk_cov_se_ard_dev(gpk_handle h, const double* dX, int n, int D, int64_t ldx, const double* theta, double* dK, int64_t ldk) {
-    if (!h || n < 0 || ldx < n || ldk < n) return gpk_set_error(h, GPK_EINVAL, "gpk_cov_se_ard: bad dimensions");
+    int rc = gpk_check_args(h, "gpk_cov_se_ard_dev", ldk >= n, n, 0, ldx, D, 0);
+    if (rc) return rc;
     CovParams cp;
-    int rc = gpk_make_cov_params(h, theta, D, 0, 0.0, &cp);
+    rc = gpk_make_cov_params(h, theta, D, 0, 0.0, &cp);
     if (rc) return rc;
     return gpk_cov_sym_full(h, dX, n, ldx, cp, dK, ldk);
 }
 
 int gpk_cov_se_ard(gpk_handle h, const double* X, int n, int D, int64_t ldx, const double* theta, double* K, int64_t ldk) {
-    if (!h || n < 0 || ldx < n || ldk < n) return gpk_set_error(h, GPK_EINVAL, "gpk_cov_se_ard: bad dimensions");
-    if (n == 0) return GPK_OK;
+    int rc = gpk_check_args(h, "gpk_cov_se_ard", ldk >= n, n, 0, ldx, D, 0);
+    if (rc || n == 0) return rc;
     GPK_CUDA(h, cudaSetDevice(h->device));
     ARENA_OR_FAIL(dX, double*, h, ARENA_X, (size_t)n * D * sizeof(double));
     ARENA_OR_FAIL(dK, double*, h, ARENA_IO, (size_t)n * n * sizeof(double));
-    int rc = gpk_upload_matrix(h, dX, X, n, D, ldx);
+    rc = gpk_upload_matrix(h, dX, X, n, D, ldx);
     if (rc) return rc;
     rc = gpk_cov_se_ard_dev(h, dX, n, D, n, theta, dK, n);
     if (rc) return rc;
@@ -208,22 +227,23 @@ int gpk_cov_se_ard(gpk_handle h, const double* X, int n, int D, int64_t ldx, con
 
 int gpk_cov_cross_se_ard_dev(gpk_handle h, const double* dX1, int m, int64_t ldx1, const double* dX2, int n, int64_t ldx2,
                              int D, const double* theta, double* dK, int64_t ldk) {
-    if (!h || m < 0 || n < 0 || ldx1 < m || ldx2 < n || ldk < m) return gpk_set_error(h, GPK_EINVAL, "gpk_cov_cross: bad dimensions");
+    int rc = gpk_check_args(h, "gpk_cov_cross_se_ard_dev", m >= 0 && ldx1 >= m && ldk >= m, n, 0, ldx2, D, 0);
+    if (rc) return rc;
     CovParams cp;
-    int rc = gpk_make_cov_params(h, theta, D, 0, 0.0, &cp);
+    rc = gpk_make_cov_params(h, theta, D, 0, 0.0, &cp);
     if (rc) return rc;
     return gpk_cov_cross(h, dX1, m, ldx1, dX2, n, ldx2, cp, dK, ldk, m, n);
 }
 
 int gpk_cov_cross_se_ard(gpk_handle h, const double* X1, int m, int64_t ldx1, const double* X2, int n, int64_t ldx2, int D,
                          const double* theta, double* K, int64_t ldk) {
-    if (!h || m < 0 || n < 0 || ldx1 < m || ldx2 < n || ldk < m) return gpk_set_error(h, GPK_EINVAL, "gpk_cov_cross: bad dimensions");
-    if (m == 0 || n == 0) return GPK_OK;
+    int rc = gpk_check_args(h, "gpk_cov_cross_se_ard", m >= 0 && ldx1 >= m && ldk >= m, n, 0, ldx2, D, 0);
+    if (rc || m == 0 || n == 0) return rc;
     GPK_CUDA(h, cudaSetDevice(h->device));
     ARENA_OR_FAIL(dX, double*, h, ARENA_X, (size_t)(m + n) * D * sizeof(double));
     ARENA_OR_FAIL(dK, double*, h, ARENA_IO, (size_t)m * n * sizeof(double));
     double* dX2 = dX + (size_t)m * D;
-    int rc = gpk_upload_matrix(h, dX, X1, m, D, ldx1);
+    rc = gpk_upload_matrix(h, dX, X1, m, D, ldx1);
     if (rc) return rc;
     rc = gpk_upload_matrix(h, dX2, X2, n, D, ldx2);
     if (rc) return rc;
@@ -236,7 +256,8 @@ int gpk_cov_cross_se_ard(gpk_handle h, const double* X1, int m, int64_t ldx1, co
 
 int gpk_cov_deriv_se_ard(gpk_handle h, int param_num, const double* X, int n, int D, int64_t ldx, const double* theta,
                          double* dKout, int64_t ldk) {
-    if (!h || n < 0 || ldx < n || ldk < n) return gpk_set_error(h, GPK_EINVAL, "gpk_cov_deriv: bad dimensions");
+    int rc = gpk_check_args(h, "gpk_cov_deriv_se_ard", ldk >= n, n, 0, ldx, D, 0);
+    if (rc) return rc;
     if (param_num < 1 || param_num > gpk_theta_len(h, D))
         return gpk_set_error(h, GPK_EINVAL, "scala.MatchError: hyper-parameter %d outside 1..%d", param_num, gpk_theta_len(h, D));
     if (n == 0) return GPK_OK;
@@ -244,7 +265,7 @@ int gpk_cov_deriv_se_ard(gpk_handle h, int param_num, const double* X, int n, in
     ARENA_OR_FAIL(dX, double*, h, ARENA_X, (size_t)n * D * sizeof(double));
     ARENA_OR_FAIL(dK, double*, h, ARENA_IO, (size_t)n * n * sizeof(double));
     CovParams cp;
-    int rc = gpk_make_cov_params(h, theta, D, 0, 0.0, &cp);
+    rc = gpk_make_cov_params(h, theta, D, 0, 0.0, &cp);
     if (rc) return rc;
     rc = gpk_upload_matrix(h, dX, X, n, D, ldx);
     if (rc) return rc;
@@ -263,15 +284,12 @@ int gpk_potrf_lower(gpk_handle h, const double* A, int n, int64_t lda, double* L
     if (n == 0) return GPK_OK;
     GPK_CUDA(h, cudaSetDevice(h->device));
     const int N = gpk_pad(n);
-    ARENA_OR_FAIL(dIn, double*, h, ARENA_IO, (size_t)n * n * sizeof(double));
     ARENA_OR_FAIL(dA, double*, h, ARENA_A, (size_t)N * N * sizeof(double));
     ARENA_OR_FAIL(dLi, double*, h, ARENA_B, (size_t)N * N * sizeof(double));
     ARENA_OR_FAIL(dT, double*, h, ARENA_T, gpk_chol_scratch_doubles(N) * sizeof(double));
-    int rc = gpk_upload_matrix(h, dIn, A, n, n, lda);
-    if (rc) return rc;
     int* d_notsym = h->d_info + 1;
     GPK_CUDA(h, cudaMemsetAsync(d_notsym, 0, sizeof(int), h->stream));
-    rc = gpk_load_sym_padded(h, dA, N, dIn, n, n, check_symmetric ? d_notsym : nullptr);
+    int rc = gpk_upload_padded(h, dA, N, A, n, lda, GPK_PAD_SYM, check_symmetric ? d_notsym : nullptr);
     if (rc) return rc;
     if (check_symmetric) {
         int ns = 0;
@@ -281,11 +299,9 @@ int gpk_potrf_lower(gpk_handle h, const double* A, int n, int64_t lda, double* L
     }
     rc = gpk_potrf_factor(h, dA, dLi, dT, N, h->d_info);     // L only: n^3/3 flops (no L^-1, no K^-1)
     if (rc) return rc;
-    rc = gpk_store_lower(h, dIn, n, dA, N, n);
-    if (rc) return rc;
     rc = gpk_finish_info(h);
     if (rc) return rc;
-    rc = gpk_download_matrix(h, L, ldl, dIn, n, n);
+    rc = gpk_download_tri(h, L, ldl, dA, N, n, 0);
     if (rc) return rc;
     return gpk_synchronize(h);
 }
@@ -295,20 +311,15 @@ int gpk_trtri(gpk_handle h, int is_upper, const double* T, int n, int64_t ldt, d
     if (n == 0) return GPK_OK;
     GPK_CUDA(h, cudaSetDevice(h->device));
     const int N = gpk_pad(n);
-    ARENA_OR_FAIL(dIn, double*, h, ARENA_IO, (size_t)n * n * sizeof(double));
     ARENA_OR_FAIL(dA, double*, h, ARENA_A, (size_t)N * N * sizeof(double));
     ARENA_OR_FAIL(dLi, double*, h, ARENA_B, (size_t)N * N * sizeof(double));
     ARENA_OR_FAIL(dT, double*, h, ARENA_T, gpk_chol_scratch_doubles(N) * sizeof(double));
-    int rc = gpk_upload_matrix(h, dIn, T, n, n, ldt);
-    if (rc) return rc;
     // an upper-triangular U is handled through its transpose: (U^t)^-1 = (U^-1)^t
-    rc = gpk_load_tri_padded(h, dA, N, dIn, n, n, is_upper ? 1 : 0);
+    int rc = gpk_upload_padded(h, dA, N, T, n, ldt, is_upper ? GPK_PAD_UPPER : GPK_PAD_LOWER);
     if (rc) return rc;
     rc = gpk_trtri_lower(h, dA, dLi, dT, N);
     if (rc) return rc;
-    rc = gpk_store_tri(h, dIn, n, dLi, N, n, is_upper ? 1 : 0);
-    if (rc) return rc;
-    rc = gpk_download_matrix(h, Tinv, ldi, dIn, n, n);
+    rc = gpk_download_tri(h, Tinv, ldi, dLi, N, n, is_upper ? 1 : 0);
     if (rc) return rc;
     return gpk_synchronize(h);
 }
@@ -368,11 +379,13 @@ int trsm_rec(gpk_handle h, const double* Lw, const double* Di, int N, int backwa
 }  // namespace
 
 // Lw: padded lower factor on the device.  Inverts its diagonal 128-blocks into Di (one launch) and substitutes.
-int gpk_trsm_padded(gpk_handle h, const double* Lw, double* Di, int N, int backward, double* B, double* X, int M) {
+int gpk_trsm_padded(gpk_handle h, const double* Lw, double* Di, int N, int backward, double* B, double* X, int M, int nvec) {
     int rc = gpk_base_potrf_trtri(h, const_cast<double*>(Lw), N, Di, GPK_TILE, h->d_info + 2, 0, 1, N / GPK_TILE,
                                   (int64_t)GPK_TILE * (N + 1), (int64_t)GPK_TILE * GPK_TILE, 0, GPK_TILE);
     if (rc) return rc;
-    return trsm_rec(h, Lw, Di, N, backward, B, X, M, 0, N);
+    if (M > 0) return trsm_rec(h, Lw, Di, N, backward, B, X, M, 0, N);
+    for (int c = 0; c < nvec && !rc; ++c) rc = trsm_rec(h, Lw, Di, N, backward, B + (size_t)c * N, X + (size_t)c * N, 0, 0, N);
+    return rc;
 }
 
 extern "C" {
@@ -387,27 +400,18 @@ int gpk_trsm(gpk_handle h, int upper, int transposed, const double* T, int n, in
     // a handful of right-hand sides go column by column through the mat-vec path (no padding to a 128-column GEMM operand)
     const bool vec = nrhs <= 4;
     const int N = gpk_pad(n), M = vec ? nrhs : gpk_pad(nrhs);
-    ARENA_OR_FAIL(dIn, double*, h, ARENA_IO, (size_t)n * n * sizeof(double));
     ARENA_OR_FAIL(dA, double*, h, ARENA_A, (size_t)N * N * sizeof(double));
     ARENA_OR_FAIL(dDi, double*, h, ARENA_T, (size_t)N * GPK_TILE * sizeof(double));
     ARENA_OR_FAIL(dB, double*, h, ARENA_IO2, (size_t)2 * N * M * sizeof(double));
     double* dX = dB + (size_t)N * M;
-    int rc = gpk_upload_matrix(h, dIn, T, n, n, ldt);
-    if (rc) return rc;
-    rc = gpk_load_tri_padded(h, dA, N, dIn, n, n, stored_upper);   // dA = lower-triangular Lw (= stored or stored^t)
+    // dA = lower-triangular Lw (= stored or stored^t)
+    int rc = gpk_upload_padded(h, dA, N, T, n, ldt, stored_upper ? GPK_PAD_UPPER : GPK_PAD_LOWER);
     if (rc) return rc;
     GPK_CUDA(h, cudaMemsetAsync(dB, 0, (size_t)2 * N * M * sizeof(double), h->stream));
     GPK_CUDA(h, cudaMemcpy2DAsync(dB, (size_t)N * sizeof(double), B, (size_t)ldb * sizeof(double), (size_t)n * sizeof(double),
                                   (size_t)nrhs, cudaMemcpyHostToDevice, h->stream));
     // effective operand E: lower (forwardSolve) -> E = Lw, X = Lw^-1 B;  upper (backSolve) -> E = Lw^t, X = Lw^-t B
-    if (vec) {
-        rc = gpk_base_potrf_trtri(h, dA, N, dDi, GPK_TILE, h->d_info + 2, 0, 1, N / GPK_TILE, (int64_t)GPK_TILE * (N + 1),
-                                  (int64_t)GPK_TILE * GPK_TILE, 0, GPK_TILE);
-        for (int c = 0; c < nrhs && !rc; ++c)
-            rc = trsm_rec(h, dA, dDi, N, upper ? 1 : 0, dB + (size_t)c * N, dX + (size_t)c * N, 0, 0, N);
-    } else {
-        rc = gpk_trsm_padded(h, dA, dDi, N, upper ? 1 : 0, dB, dX, M);
-    }
+    rc = gpk_trsm_padded(h, dA, dDi, N, upper ? 1 : 0, dB, dX, vec ? 0 : M, nrhs);
     if (rc) return rc;
     GPK_CUDA(h, cudaMemcpy2DAsync(Xout, (size_t)ldx * sizeof(double), dX, (size_t)N * sizeof(double), (size_t)n * sizeof(double),
                                   (size_t)nrhs, cudaMemcpyDeviceToHost, h->stream));
@@ -426,18 +430,18 @@ int gpk_potrf_lower_dev(gpk_handle h, double* dA, int n, int64_t lda, int* info_
     const bool in_place = N == n && lda == n && !((uintptr_t)dA & 15);
     double* dW = dA;
     if (!in_place) {
-        dW = (double*)gpk_arena(h, ARENA_A, (size_t)N * N * sizeof(double));
-        if (!dW) return gpk_set_error(h, GPK_ENOMEM, "device allocation failed");
+        ARENA_OR_FAIL(dWork, double*, h, ARENA_A, (size_t)N * N * sizeof(double));
+        dW = dWork;
     }
     // ~40 launches per block column, most of them small and dependent: a caller that factors the same buffer again (a solver in a
     // loop) replays the launch sequence from a graph, like the evaluation and the EP sweep -- up to N = 4096, where the launch gaps
     // dominate (2.74 -> 2.45 ms at n = 4096; at n = 8192 replay is SLOWER, 8.77 -> 9.27 ms: profiles/r02_potrf_nb.log)
     auto body = [&]() {
         int rc = GPK_OK;
-        if (!in_place) rc = gpk_load_sym_padded(h, dW, N, dA, n, lda, nullptr);
+        if (!in_place) rc = gpk_load_padded(h, dW, N, dA, n, lda, GPK_PAD_SYM);
         if (!rc) rc = gpk_potrf_factor(h, dW, dLi, dT, N, info);
-        if (!rc) rc = in_place ? gpk_store_lower(h, dA, n, dA, N, n)     // zero the strict upper triangle (element-wise, in place)
-                               : gpk_store_lower(h, dA, lda, dW, N, n);
+        if (!rc) rc = in_place ? gpk_store_tri(h, dA, n, dA, N, n, 0)     // zero the strict upper triangle (element-wise, in place)
+                               : gpk_store_tri(h, dA, lda, dW, N, n, 0);
         return rc;
     };
     if (!h->graph_mode || N < 1024 || N > 4096) return body();

@@ -195,7 +195,6 @@ int gpk_make_problem_params(gpk_handle h, const double* theta, int D, int has_si
 }
 
 int gpk_make_cov_params(gpk_handle h, const double* theta, int D, int has_sigma_noise, double sigma_noise, CovParams* out) {
-    if (D < 1 || D > GPK_MAX_D) return gpk_set_error(h, GPK_EINVAL, "feature dimension D=%d outside 1..%d", D, GPK_MAX_D);
     memset(out, 0, sizeof(*out));
     out->D = D;
     out->kind = h ? h->kernel_family : GPK_KERNEL_SE_ARD;

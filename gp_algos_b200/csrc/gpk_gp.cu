@@ -13,10 +13,6 @@
 
 namespace {
 
-#define ARENA_OR_FAIL(ptr, type, h, which, bytes)           \
-    type ptr = (type)gpk_arena((h), (which), (bytes));      \
-    if (!ptr) return GPK_ENOMEM
-
 size_t batch_budget_bytes() {
     static size_t v = 0;
     if (!v) {
@@ -50,14 +46,14 @@ int make_work(gpk_handle h, int n, int D, int Bwant, Work* w) {
     int B = Bwant;
     if ((size_t)B * per > batch_budget_bytes()) B = (int)(batch_budget_bytes() / per);
     if (B < 1) B = 1;
+    ARENA_OR_FAIL(A, double*, h, ARENA_A, (size_t)B * N * N * sizeof(double));
+    ARENA_OR_FAIL(Li, double*, h, ARENA_B, (size_t)B * N * N * sizeof(double));
+    ARENA_OR_FAIL(T, double*, h, ARENA_T, (size_t)B * sT * sizeof(double));
+    ARENA_OR_FAIL(m, double*, h, ARENA_MISC, (size_t)B * ((size_t)3 * N + sScr) * sizeof(double));
+    ARENA_OR_FAIL(pp_dev, ProblemParams*, h, ARENA_PP, (size_t)B * sizeof(ProblemParams));
+    ARENA_OR_FAIL(info_dev, int*, h, ARENA_INFO, (size_t)B * sizeof(int));
     w->N = N; w->B = B; w->sT = sT; w->sScratch = sScr;
-    w->A = (double*)gpk_arena(h, ARENA_A, (size_t)B * N * N * sizeof(double));
-    w->Li = (double*)gpk_arena(h, ARENA_B, (size_t)B * N * N * sizeof(double));
-    w->T = (double*)gpk_arena(h, ARENA_T, (size_t)B * sT * sizeof(double));
-    double* m = (double*)gpk_arena(h, ARENA_MISC, (size_t)B * ((size_t)3 * N + sScr) * sizeof(double));
-    w->pp_dev = (ProblemParams*)gpk_arena(h, ARENA_PP, (size_t)B * sizeof(ProblemParams));
-    w->info_dev = (int*)gpk_arena(h, ARENA_INFO, (size_t)B * sizeof(int));
-    if (!w->A || !w->Li || !w->T || !m || !w->pp_dev || !w->info_dev) return GPK_ENOMEM;
+    w->A = A; w->Li = Li; w->T = T; w->pp_dev = pp_dev; w->info_dev = info_dev;
     w->ypad = m;
     w->z = m + (size_t)B * N;
     w->alpha = m + (size_t)2 * B * N;
@@ -127,8 +123,8 @@ int nll_grad_core(gpk_handle h, int B, const double* dX, int n, int D, int64_t l
         int* info = info_dev ? info_dev + b0 : (B == 1 ? h->d_info : w.info_dev);
         double* Kinv = nullptr;
         if (nparams > 0 && gpk_use_pipelined(w.N, bc)) {
-            Kinv = (double*)gpk_arena(h, ARENA_KINV, (size_t)w.N * w.N * sizeof(double));
-            if (!Kinv) return GPK_ENOMEM;
+            ARENA_OR_FAIL(dKinv, double*, h, ARENA_KINV, (size_t)w.N * w.N * sizeof(double));
+            Kinv = dKinv;
         }
         cudaEvent_t kinv_done = nullptr;
         rc = fit_core(h, w, bc, X, n, D, ldx, strideX, dy + (size_t)b0 * n, pp0, 0, w.Li, w.alpha, out_dev + b0 * so, so, info, Kinv,
@@ -148,6 +144,41 @@ int nll_grad_core(gpk_handle h, int B, const double* dX, int n, int D, int64_t l
     return GPK_OK;
 }
 
+// A stack of nx host matrices (n x D, ld ldx, matrix b at X + b*stride) to the device, compact and back to back (matrix b at
+// dst + b*n*D): one copy when the stack already is laid out so (Breeze matrices back to back)
+int upload_stack(gpk_handle h, double* dst, const double* X, int nx, int n, int D, int64_t ldx, int64_t stride) {
+    if (ldx == n && (nx == 1 || stride == (int64_t)n * D)) {
+        GPK_CUDA(h, cudaMemcpyAsync(dst, X, (size_t)nx * n * D * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+        return GPK_OK;
+    }
+    int rc = GPK_OK;
+    for (int b = 0; b < nx && !rc; ++b) rc = gpk_upload_matrix(h, dst + (size_t)b * n * D, X + b * stride, n, D, ldx);
+    return rc;
+}
+
+// The results of a batched call come back through the handle's pinned staging (grown on demand, never per call): res_bytes
+// of results at dres (0: none) followed on the device by the B per-problem info words, staged at h->res_pinned in one copy
+// and one synchronisation.  info (optional) receives the info words.  The call's first failure goes to h->last_info and
+// sets *failed, which stays set across the chunks of one call: GPK_ENOTPD from then on.
+int fetch_batch_results(gpk_handle h, const void* dres, size_t res_bytes, int B, int* info, bool* failed) {
+    const size_t bytes = res_bytes + (size_t)B * sizeof(int);
+    if (h->res_pinned_bytes < bytes) {
+        if (h->res_pinned) cudaFreeHost(h->res_pinned);
+        h->res_pinned = nullptr; h->res_pinned_bytes = 0;
+        if (cudaMallocHost(&h->res_pinned, bytes) != cudaSuccess) { cudaGetLastError(); return gpk_set_error(h, GPK_ENOMEM, "pinned host allocation failed"); }
+        h->res_pinned_bytes = bytes;
+    }
+    GPK_CUDA(h, cudaMemcpyAsync(h->res_pinned, dres, bytes, cudaMemcpyDeviceToHost, h->stream));
+    GPK_CUDA(h, cudaStreamSynchronize(h->stream));
+    const int* hinfo = (const int*)((const char*)h->res_pinned + res_bytes);
+    for (int b = 0; b < B; ++b) {
+        if (info) info[b] = hinfo[b];
+        if (hinfo[b] && !*failed) { *failed = true; h->last_info = hinfo[b]; }
+    }
+    if (*failed) return gpk_set_error(h, GPK_ENOTPD, "at least one problem of the batch is not positive definite (see info[])");
+    return GPK_OK;
+}
+
 __global__ void store_params_kernel(const ProblemParams pp, ProblemParams* __restrict__ dst) {
     if (threadIdx.x == 0) *dst = pp;
 }
@@ -163,7 +194,9 @@ int nll_grad_single(gpk_handle h, const double* dX, int n, int D, int64_t ldx, c
     Work w;
     rc = make_work(h, n, D, 1, &w);     // sizes every arena now, so that the workspace epoch the cache compares is final
     if (rc) return rc;
-    if (nparams > 0 && gpk_use_pipelined(w.N, 1) && !gpk_arena(h, ARENA_KINV, (size_t)w.N * w.N * sizeof(double))) return GPK_ENOMEM;
+    if (nparams > 0 && gpk_use_pipelined(w.N, 1)) {
+        ARENA_OR_FAIL(Kinv, double*, h, ARENA_KINV, (size_t)w.N * w.N * sizeof(double));
+    }
     GraphKey key;
     memset(&key, 0, sizeof(key));
     key.p[0] = dX; key.p[1] = dy; key.p[2] = out_dev; key.p[3] = info_dev;
@@ -221,6 +254,35 @@ namespace {
 int upload_model_x(gpk_handle h, gpk_model m, const double* X, int64_t ldx) {   // host n x D (ld ldx) -> device (ld m->ldx)
     GPK_CUDA(h, cudaMemcpy2DAsync(m->X, (size_t)m->ldx * sizeof(double), X, (size_t)ldx * sizeof(double), (size_t)m->n * sizeof(double),
                                   (size_t)m->D, cudaMemcpyHostToDevice, h->stream));
+    return GPK_OK;
+}
+
+// The three device buffers of a model of padded size N: X (N x D), Li (N x N), alpha (N) -- all three or none
+int model_buffers(gpk_handle h, int N, int D, double** X, double** Li, double** alpha) {
+    *X = *Li = *alpha = nullptr;
+    if (cudaMalloc((void**)X, (size_t)N * D * sizeof(double)) == cudaSuccess &&
+        cudaMalloc((void**)Li, (size_t)N * N * sizeof(double)) == cudaSuccess &&
+        cudaMalloc((void**)alpha, (size_t)N * sizeof(double)) == cudaSuccess)
+        return GPK_OK;
+    cudaGetLastError();
+    cudaFree(*X); cudaFree(*Li); cudaFree(*alpha);
+    *X = *Li = *alpha = nullptr;
+    return gpk_set_error(h, GPK_ENOMEM, "allocation of a model of padded size %d failed", N);
+}
+
+// A new resident model of n training rows whose buffers `fill` writes; a failure destroys the half-built model here.
+template <class F>
+int model_make(gpk_handle h, int n, int D, const double* theta, gpk_model* out, F&& fill) {
+    GPK_CUDA(h, cudaSetDevice(h->device));
+    gpk_model m = new (std::nothrow) gpk_model_s();
+    if (!m) return GPK_ENOMEM;
+    memset(m, 0, sizeof(*m));
+    m->n = n; m->N = gpk_pad(n); m->D = D; m->ldx = m->N;
+    memcpy(m->theta, theta, sizeof(double) * gpk_theta_len(h, D));
+    int rc = model_buffers(h, m->N, D, &m->X, &m->Li, &m->alpha);
+    if (!rc) rc = fill(m);
+    if (rc) { gpk_gp_model_destroy(h, m); return rc; }
+    *out = m;
     return GPK_OK;
 }
 
@@ -285,24 +347,23 @@ extern "C" {
 // ------------------------------------------------------------------------------------------------
 int gpk_gp_nll_grad_dev(gpk_handle h, const double* dX, int n, int D, int64_t ldx, const double* dy, const double* theta,
                         int has_s, double s, int nparams, double* out_dev, int* info_dev) {
-    if (!h || n <= 0 || ldx < n) return gpk_set_error(h, GPK_EINVAL, "gpk_gp_nll_grad: bad dimensions");
-    if (D < 1 || D > GPK_MAX_D) return gpk_set_error(h, GPK_EINVAL, "feature dimension D=%d outside 1..%d", D, GPK_MAX_D);
-    if (nparams < 0 || nparams > gpk_theta_len(h, D)) return gpk_set_error(h, GPK_EINVAL, "nparams=%d outside 0..%d", nparams, gpk_theta_len(h, D));
+    int rc = gpk_check_args(h, "gpk_gp_nll_grad_dev", true, n, 1, ldx, D, nparams);
+    if (rc) return rc;
     return nll_grad_single(h, dX, n, D, ldx, dy, theta, has_s, s, nparams, out_dev, info_dev);
 }
 
 int gpk_gp_nll_grad(gpk_handle h, const double* X, int n, int D, int64_t ldx, const double* y, const double* theta,
                     int has_s, double s, int nparams, double* ll, double* grad) {
-    if (!h || n <= 0 || ldx < n) return gpk_set_error(h, GPK_EINVAL, "gpk_gp_nll_grad: bad dimensions (require rows == targets)");
-    if (D < 1 || D > GPK_MAX_D) return gpk_set_error(h, GPK_EINVAL, "feature dimension D=%d outside 1..%d", D, GPK_MAX_D);
+    int rc = gpk_check_args(h, "gpk_gp_nll_grad", true, n, 1, ldx, D, nparams);
+    if (rc) return rc;
     GPK_CUDA(h, cudaSetDevice(h->device));
     ARENA_OR_FAIL(dX, double*, h, ARENA_X, ((size_t)n * D + n + 256) * sizeof(double));
     double* dy = dX + (size_t)n * D;
     double* dout = dy + n;
-    int rc = gpk_upload_matrix(h, dX, X, n, D, ldx);
+    rc = gpk_upload_matrix(h, dX, X, n, D, ldx);
     if (rc) return rc;
     GPK_CUDA(h, cudaMemcpyAsync(dy, y, (size_t)n * sizeof(double), cudaMemcpyHostToDevice, h->stream));
-    rc = gpk_gp_nll_grad_dev(h, dX, n, D, n, dy, theta, has_s, s, nparams, dout, nullptr);
+    rc = nll_grad_single(h, dX, n, D, n, dy, theta, has_s, s, nparams, dout, nullptr);
     if (rc) return rc;
     GPK_CUDA(h, cudaMemcpyAsync(h->h_pinned, dout, (size_t)(nparams + 1) * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
     rc = gpk_finish_info(h);
@@ -315,15 +376,15 @@ int gpk_gp_nll_grad(gpk_handle h, const double* X, int n, int D, int64_t ldx, co
 int gpk_gp_nll_grad_batched_dev(gpk_handle h, int B, const double* dX, int n, int D, int64_t ldx, int64_t strideX,
                                 const double* dy, const double* thetas, int has_s, double s, int nparams, double* out_dev,
                                 int* info_dev) {
-    if (!h || B <= 0 || n <= 0 || ldx < n || !info_dev) return gpk_set_error(h, GPK_EINVAL, "gpk_gp_nll_grad_batched: bad arguments");
-    if (D < 1 || D > GPK_MAX_D) return gpk_set_error(h, GPK_EINVAL, "feature dimension D=%d outside 1..%d", D, GPK_MAX_D);
-    if (nparams < 0 || nparams > gpk_theta_len(h, D)) return gpk_set_error(h, GPK_EINVAL, "nparams=%d outside 0..%d", nparams, gpk_theta_len(h, D));
+    int rc = gpk_check_args(h, "gpk_gp_nll_grad_batched_dev", B > 0 && info_dev, n, 1, ldx, D, nparams);
+    if (rc) return rc;
     return nll_grad_core(h, B, dX, n, D, ldx, strideX, dy, thetas, has_s, s, nparams, out_dev, info_dev);
 }
 
 int gpk_gp_nll_grad_batched(gpk_handle h, int B, const double* X, int n, int D, int64_t ldx, int64_t strideX, const double* y,
                             const double* thetas, int has_s, double s, int nparams, double* ll, double* grad, int* info) {
-    if (!h || B <= 0 || n <= 0 || ldx < n) return gpk_set_error(h, GPK_EINVAL, "gpk_gp_nll_grad_batched: bad arguments");
+    int rc = gpk_check_args(h, "gpk_gp_nll_grad_batched", B > 0, n, 1, ldx, D, nparams);
+    if (rc) return rc;
     if (strideX != 0 && strideX < (int64_t)ldx * (D - 1) + n)
         return gpk_set_error(h, GPK_EINVAL, "gpk_gp_nll_grad_batched: strideX overlaps consecutive problems");
     GPK_CUDA(h, cudaSetDevice(h->device));
@@ -333,38 +394,20 @@ int gpk_gp_nll_grad_batched(gpk_handle h, int B, const double* X, int n, int D, 
     double* dy = dX + (size_t)nx * n * D;
     double* dout = dy + (size_t)B * n;
     int* dinfo = (int*)(dout + B * so);
-    int rc = GPK_OK;
-    if (ldx == n && (nx == 1 || strideX == (int64_t)n * D)) {
-        // the stack is one contiguous block (Breeze matrices laid out back to back): a single copy
-        GPK_CUDA(h, cudaMemcpyAsync(dX, X, (size_t)nx * n * D * sizeof(double), cudaMemcpyHostToDevice, h->stream));
-    } else {
-        for (int b = 0; b < nx && !rc; ++b) rc = gpk_upload_matrix(h, dX + (size_t)b * n * D, X + b * strideX, n, D, ldx);
-        if (rc) return rc;
-    }
-    GPK_CUDA(h, cudaMemcpyAsync(dy, y, (size_t)B * n * sizeof(double), cudaMemcpyHostToDevice, h->stream));
-    rc = gpk_gp_nll_grad_batched_dev(h, B, dX, n, D, n, strideX ? (int64_t)n * D : 0, dy, thetas, has_s, s, nparams, dout, dinfo);
+    rc = upload_stack(h, dX, X, nx, n, D, ldx, strideX);
     if (rc) return rc;
-    // results come back through the handle's pinned staging buffer (grown on demand, never per call)
-    const size_t res_bytes = B * so * sizeof(double) + (size_t)B * sizeof(int);
-    if (h->res_pinned_bytes < res_bytes) {
-        if (h->res_pinned) cudaFreeHost(h->res_pinned);
-        h->res_pinned = nullptr; h->res_pinned_bytes = 0;
-        if (cudaMallocHost(&h->res_pinned, res_bytes) != cudaSuccess) { cudaGetLastError(); return gpk_set_error(h, GPK_ENOMEM, "pinned host allocation failed"); }
-        h->res_pinned_bytes = res_bytes;
-    }
-    double* hout = (double*)h->res_pinned;
-    int* hinfo = (int*)(hout + B * so);
-    GPK_CUDA(h, cudaMemcpyAsync(hout, dout, res_bytes, cudaMemcpyDeviceToHost, h->stream));   // dinfo follows dout on the device too
-    GPK_CUDA(h, cudaStreamSynchronize(h->stream));
-    int bad = 0;
+    GPK_CUDA(h, cudaMemcpyAsync(dy, y, (size_t)B * n * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    rc = nll_grad_core(h, B, dX, n, D, n, strideX ? (int64_t)n * D : 0, dy, thetas, has_s, s, nparams, dout, dinfo);
+    if (rc) return rc;
+    bool failed = false;
+    rc = fetch_batch_results(h, dout, B * so * sizeof(double), B, info, &failed);   // dinfo follows dout
+    if (rc && rc != GPK_ENOTPD) return rc;
+    const double* hout = (const double*)h->res_pinned;
     for (int b = 0; b < B; ++b) {
         ll[b] = hout[b * so];
         for (int p = 0; p < nparams; ++p) grad[(size_t)b * nparams + p] = hout[b * so + 1 + p];
-        if (info) info[b] = hinfo[b];
-        if (hinfo[b] && !bad) { bad = 1; h->last_info = hinfo[b]; }
     }
-    if (bad) return gpk_set_error(h, GPK_ENOTPD, "at least one problem of the batch is not positive definite (see info[])");
-    return GPK_OK;
+    return rc;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -372,13 +415,13 @@ int gpk_gp_nll_grad_batched(gpk_handle h, int B, const double* X, int n, int D, 
 // ------------------------------------------------------------------------------------------------
 int gpk_gp_fit(gpk_handle h, const double* X, int n, int D, int64_t ldx, const double* y, const double* theta, int has_s,
                double s, double* L, int64_t ldl, double* alpha, double* ll) {
-    if (!h || n <= 0 || ldx < n || (L && ldl < n)) return gpk_set_error(h, GPK_EINVAL, "gpk_gp_fit: bad dimensions");
-    if (D < 1 || D > GPK_MAX_D) return gpk_set_error(h, GPK_EINVAL, "feature dimension D=%d outside 1..%d", D, GPK_MAX_D);
+    int rc = gpk_check_args(h, "gpk_gp_fit", !L || ldl >= n, n, 1, ldx, D, 0);
+    if (rc) return rc;
     GPK_CUDA(h, cudaSetDevice(h->device));
     ARENA_OR_FAIL(dX, double*, h, ARENA_X, ((size_t)n * D + n + 256) * sizeof(double));
     double* dy = dX + (size_t)n * D;
     double* dout = dy + n;
-    int rc = gpk_upload_matrix(h, dX, X, n, D, ldx);
+    rc = gpk_upload_matrix(h, dX, X, n, D, ldx);
     if (rc) return rc;
     GPK_CUDA(h, cudaMemcpyAsync(dy, y, (size_t)n * sizeof(double), cudaMemcpyHostToDevice, h->stream));
     Work w;
@@ -395,10 +438,7 @@ int gpk_gp_fit(gpk_handle h, const double* X, int n, int D, int64_t ldx, const d
     if (ll) *ll = h->h_pinned[0];
     if (alpha) GPK_CUDA(h, cudaMemcpyAsync(alpha, w.alpha, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
     if (L) {
-        ARENA_OR_FAIL(dOut, double*, h, ARENA_IO, (size_t)n * n * sizeof(double));
-        rc = gpk_store_lower(h, dOut, n, w.A, w.N, n);
-        if (rc) return rc;
-        rc = gpk_download_matrix(h, L, ldl, dOut, n, n);
+        rc = gpk_download_tri(h, L, ldl, w.A, w.N, n, 0);
         if (rc) return rc;
     }
     return gpk_synchronize(h);
@@ -407,26 +447,6 @@ int gpk_gp_fit(gpk_handle h, const double* X, int n, int D, int64_t ldx, const d
 // ------------------------------------------------------------------------------------------------
 // resident model + prediction
 // ------------------------------------------------------------------------------------------------
-static int model_alloc(gpk_handle h, int n, int D, const double* theta, gpk_model* out) {
-    gpk_model m = new (std::nothrow) gpk_model_s();
-    if (!m) return GPK_ENOMEM;
-    memset(m, 0, sizeof(*m));
-    m->n = n; m->N = gpk_pad(n); m->D = D; m->ldx = m->N;
-    memcpy(m->theta, theta, sizeof(double) * gpk_theta_len(h, D));
-    if (cudaMalloc((void**)&m->X, (size_t)m->ldx * D * sizeof(double)) != cudaSuccess ||
-        cudaMalloc((void**)&m->Li, (size_t)m->N * m->N * sizeof(double)) != cudaSuccess ||
-        cudaMalloc((void**)&m->alpha, (size_t)m->N * sizeof(double)) != cudaSuccess) {
-        cudaGetLastError();
-        if (m->X) cudaFree(m->X);
-        if (m->Li) cudaFree(m->Li);
-        if (m->alpha) cudaFree(m->alpha);
-        delete m;
-        return gpk_set_error(h, GPK_ENOMEM, "model allocation failed (n=%d)", n);
-    }
-    *out = m;
-    return GPK_OK;
-}
-
 int gpk_gp_model_destroy(gpk_handle h, gpk_model m) {
     if (!m) return GPK_OK;
     if (h) { cudaSetDevice(h->device); cudaStreamSynchronize(h->stream); }
@@ -437,58 +457,50 @@ int gpk_gp_model_destroy(gpk_handle h, gpk_model m) {
 
 int gpk_gp_model_fit(gpk_handle h, const double* X, int n, int D, int64_t ldx, const double* y, const double* theta,
                      int has_s, double s, gpk_model* out, double* ll) {
-    if (!h || !out || n <= 0 || ldx < n) return gpk_set_error(h, GPK_EINVAL, "gpk_gp_model_fit: bad dimensions");
-    if (D < 1 || D > GPK_MAX_D) return gpk_set_error(h, GPK_EINVAL, "feature dimension D=%d outside 1..%d", D, GPK_MAX_D);
-    GPK_CUDA(h, cudaSetDevice(h->device));
-    gpk_model m = nullptr;
-    int rc = model_alloc(h, n, D, theta, &m);
+    int rc = gpk_check_args(h, "gpk_gp_model_fit", out != nullptr, n, 1, ldx, D, 0);
     if (rc) return rc;
-    double* dy = (double*)gpk_arena(h, ARENA_X, ((size_t)n + 256) * sizeof(double));
-    if (!dy) rc = GPK_ENOMEM;
-    double* dout = dy + n;
-    if (!rc) rc = upload_model_x(h, m, X, ldx);
-    if (!rc) rc = (cudaMemcpyAsync(dy, y, (size_t)n * sizeof(double), cudaMemcpyHostToDevice, h->stream) == cudaSuccess) ? 0 : GPK_ECUDA;
-    Work w;
-    if (!rc) rc = make_work(h, n, D, 1, &w);
-    if (!rc) rc = gpk_make_problem_params(h, theta, D, has_s, s, &m->pp);
-    // factor straight into the model's resident buffers
-    if (!rc) rc = fit_core(h, w, 1, m->X, n, D, m->ldx, 0, dy, m->pp, 0, m->Li, m->alpha, dout, 1, h->d_info);
-    if (!rc) rc = (cudaMemcpyAsync(h->h_pinned, dout, sizeof(double), cudaMemcpyDeviceToHost, h->stream) == cudaSuccess) ? 0 : GPK_ECUDA;
-    if (!rc) rc = gpk_finish_info(h);
-    if (rc) { gpk_gp_model_destroy(h, m); return rc; }
-    // predictions never include the Option sigmaNoise in the kernel (GpPredictor.scala:31,36 use newKernelFunc only)
-    m->pp.cp.extra_diag = 0.0;
-    m->has_s = has_s ? 1 : 0; m->s = has_s ? s : 0.0;     // remembered for gpk_gp_model_append
-    if (ll) *ll = h->h_pinned[0];
-    *out = m;
-    return GPK_OK;
+    return model_make(h, n, D, theta, out, [&](gpk_model m) -> int {
+        ARENA_OR_FAIL(dy, double*, h, ARENA_X, ((size_t)n + 256) * sizeof(double));
+        double* dout = dy + n;
+        int rc = upload_model_x(h, m, X, ldx);
+        if (rc) return rc;
+        GPK_CUDA(h, cudaMemcpyAsync(dy, y, (size_t)n * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+        Work w;
+        rc = make_work(h, n, D, 1, &w);
+        if (!rc) rc = gpk_make_problem_params(h, theta, D, has_s, s, &m->pp);
+        // factor straight into the model's resident buffers
+        if (!rc) rc = fit_core(h, w, 1, m->X, n, D, m->ldx, 0, dy, m->pp, 0, m->Li, m->alpha, dout, 1, h->d_info);
+        if (rc) return rc;
+        GPK_CUDA(h, cudaMemcpyAsync(h->h_pinned, dout, sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+        rc = gpk_finish_info(h);
+        if (rc) return rc;
+        // predictions never include the Option sigmaNoise in the kernel (GpPredictor.scala:31,36 use newKernelFunc only)
+        m->pp.cp.extra_diag = 0.0;
+        m->has_s = has_s ? 1 : 0; m->s = has_s ? s : 0.0;     // remembered for gpk_gp_model_append
+        if (ll) *ll = h->h_pinned[0];
+        return GPK_OK;
+    });
 }
 
 int gpk_gp_model_from_factor(gpk_handle h, const double* X, int n, int D, int64_t ldx, const double* L, int64_t ldl,
                              const double* alpha, const double* theta, gpk_model* out) {
-    if (!h || !out || n <= 0 || ldx < n || ldl < n) return gpk_set_error(h, GPK_EINVAL, "gpk_gp_model_from_factor: bad dimensions");
-    if (D < 1 || D > GPK_MAX_D) return gpk_set_error(h, GPK_EINVAL, "feature dimension D=%d outside 1..%d", D, GPK_MAX_D);
-    GPK_CUDA(h, cudaSetDevice(h->device));
-    gpk_model m = nullptr;
-    int rc = model_alloc(h, n, D, theta, &m);
+    int rc = gpk_check_args(h, "gpk_gp_model_from_factor", out && ldl >= n, n, 1, ldx, D, 0);
     if (rc) return rc;
-    const int N = m->N;
-    rc = gpk_make_problem_params(h, theta, D, 0, 0.0, &m->pp);
-    double* dIn = (double*)gpk_arena(h, ARENA_IO, (size_t)n * n * sizeof(double));
-    double* dA = (double*)gpk_arena(h, ARENA_A, (size_t)N * N * sizeof(double));
-    double* dT = (double*)gpk_arena(h, ARENA_T, gpk_chol_scratch_doubles(N) * sizeof(double));
-    if (!dIn || !dA || !dT) rc = GPK_ENOMEM;
-    if (!rc) rc = upload_model_x(h, m, X, ldx);
-    if (!rc) rc = gpk_upload_matrix(h, dIn, L, n, n, ldl);
-    if (!rc) rc = gpk_load_tri_padded(h, dA, N, dIn, n, n, 0);
-    if (!rc) rc = gpk_trtri_lower(h, dA, m->Li, dT, N);
-    if (!rc) rc = (cudaMemsetAsync(m->alpha, 0, (size_t)N * sizeof(double), h->stream) == cudaSuccess) ? 0 : GPK_ECUDA;
-    if (!rc) rc = (cudaMemcpyAsync(m->alpha, alpha, (size_t)n * sizeof(double), cudaMemcpyHostToDevice, h->stream) == cudaSuccess) ? 0 : GPK_ECUDA;
-    if (!rc) rc = gpk_synchronize(h);
-    if (rc) { gpk_gp_model_destroy(h, m); return rc; }
-    m->has_s = -1;                                         // unknown: the caller's factor may or may not include a sigmaNoise
-    *out = m;
-    return GPK_OK;
+    return model_make(h, n, D, theta, out, [&](gpk_model m) -> int {
+        const int N = m->N;
+        int rc = gpk_make_problem_params(h, theta, D, 0, 0.0, &m->pp);
+        if (rc) return rc;
+        ARENA_OR_FAIL(dA, double*, h, ARENA_A, (size_t)N * N * sizeof(double));
+        ARENA_OR_FAIL(dT, double*, h, ARENA_T, gpk_chol_scratch_doubles(N) * sizeof(double));
+        rc = upload_model_x(h, m, X, ldx);
+        if (!rc) rc = gpk_upload_padded(h, dA, N, L, n, ldl, GPK_PAD_LOWER);
+        if (!rc) rc = gpk_trtri_lower(h, dA, m->Li, dT, N);
+        if (rc) return rc;
+        GPK_CUDA(h, cudaMemsetAsync(m->alpha, 0, (size_t)N * sizeof(double), h->stream));
+        GPK_CUDA(h, cudaMemcpyAsync(m->alpha, alpha, (size_t)n * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+        m->has_s = -1;                                     // unknown: the caller's factor may or may not include a sigmaNoise
+        return gpk_synchronize(h);
+    });
 }
 
 // gp/optimization/GPOptimizer.scala:48-71: every outer GP-UCB iteration appends ONE evaluated point to the training set and
@@ -504,16 +516,9 @@ int gpk_gp_model_append(gpk_handle h, gpk_model m, const double* x_new, double y
     const int D = m->D;
     if (m->n == m->N) {   // no padding row left: move to a factor that is one tile larger
         const int N2 = m->N + GPK_TILE;
-        double *Ln = nullptr, *an = nullptr, *Xn = nullptr;
-        if (cudaMalloc((void**)&Ln, (size_t)N2 * N2 * sizeof(double)) != cudaSuccess ||
-            cudaMalloc((void**)&an, (size_t)N2 * sizeof(double)) != cudaSuccess ||
-            cudaMalloc((void**)&Xn, (size_t)N2 * D * sizeof(double)) != cudaSuccess) {
-            cudaGetLastError();
-            if (Ln) cudaFree(Ln);
-            if (an) cudaFree(an);
-            if (Xn) cudaFree(Xn);
-            return gpk_set_error(h, GPK_ENOMEM, "model growth failed (n=%d)", m->n);
-        }
+        double *Xn, *Ln, *an;
+        int rc = model_buffers(h, N2, D, &Xn, &Ln, &an);
+        if (rc) return rc;
         model_grow_kernel<<<(unsigned)(((int64_t)N2 * N2 + 255) / 256), 256, 0, h->stream>>>(m->Li, m->N, Ln, N2);
         GPK_LAUNCH_CHECK(h);
         GPK_CUDA(h, cudaMemsetAsync(an, 0, (size_t)N2 * sizeof(double), h->stream));
@@ -715,8 +720,10 @@ int gpk_gp_models_mean_var(gpk_handle h, const gpk_model* models, int nmodels, c
 
 int gpk_gp_predict(gpk_handle h, const double* X, int n, int D, int64_t ldx, const double* y, const double* Xs, int ms,
                    int64_t ldxs, const double* theta, int has_s, double s, double* mean, double* sigma, int64_t lds, double* ll) {
+    int rc = gpk_check_args(h, "gpk_gp_predict", ms > 0 && ldxs >= ms && (!sigma || lds >= ms), n, 1, ldx, D, 0);
+    if (rc) return rc;
     gpk_model m = nullptr;
-    int rc = gpk_gp_model_fit(h, X, n, D, ldx, y, theta, has_s, s, &m, ll);
+    rc = gpk_gp_model_fit(h, X, n, D, ldx, y, theta, has_s, s, &m, ll);
     if (rc) return rc;
     rc = gpk_gp_model_predict(h, m, Xs, ms, ldxs, 1, mean, sigma, lds, nullptr, 0);
     gpk_gp_model_destroy(h, m);
@@ -731,12 +738,12 @@ int gpk_gp_predict(gpk_handle h, const double* X, int n, int D, int64_t ldx, con
 int gpk_gp_predict_batched(gpk_handle h, int B, const double* X, int n, int D, int64_t ldx, int64_t strideX, const double* y,
                            const double* thetas, const double* Xs, int ms, int64_t ldxs, int64_t strideXs, int has_s, double s,
                            double* mean, double* var, double* ll, int* info) {
-    if (!h || B <= 0 || n <= 0 || ms <= 0 || ldx < n || ldxs < ms) return gpk_set_error(h, GPK_EINVAL, "gpk_gp_predict_batched: bad arguments");
-    if (D < 1 || D > GPK_MAX_D) return gpk_set_error(h, GPK_EINVAL, "feature dimension D=%d outside 1..%d", D, GPK_MAX_D);
+    int rc = gpk_check_args(h, "gpk_gp_predict_batched", B > 0 && ms > 0 && ldxs >= ms, n, 1, ldx, D, 0);
+    if (rc) return rc;
     GPK_CUDA(h, cudaSetDevice(h->device));
     const int N = gpk_pad(n), M = gpk_pad(ms);
     Work w;
-    int rc = make_work(h, n, D, B, &w);
+    rc = make_work(h, n, D, B, &w);
     if (rc) return rc;
     const int Bc = w.B;
     const int nx = strideX ? Bc : 1, nxs = strideXs ? Bc : 1;
@@ -749,45 +756,34 @@ int gpk_gp_predict_batched(gpk_handle h, int B, const double* X, int n, int D, i
     double* dV = dKsT + (size_t)Bc * N * M;
     double* dMean = dV + (size_t)Bc * N * M;
     double* dVar = dMean + (size_t)Bc * M;
-    int* hinfo = (int*)malloc((size_t)B * sizeof(int));
-    if (!hinfo) return gpk_set_error(h, GPK_ENOMEM, "host allocation failed");
-    int bad = 0;
-    for (int b0 = 0; b0 < B && !rc; b0 += Bc) {
+    bool failed = false;
+    for (int b0 = 0; b0 < B; b0 += Bc) {
         const int bc = (B - b0 < Bc) ? B - b0 : Bc;
         ProblemParams pp0;
         rc = stage_params(h, thetas + (size_t)b0 * gpk_theta_len(h, D), D, has_s, s, bc, w.pp_dev, &pp0);
-        for (int b = 0; b < (strideX ? bc : 1) && !rc; ++b)
-            rc = gpk_upload_matrix(h, dX + (size_t)b * n * D, X + (strideX ? (b0 + b) * strideX : 0), n, D, ldx);
-        for (int b = 0; b < (strideXs ? bc : 1) && !rc; ++b)
-            rc = gpk_upload_matrix(h, dXs + (size_t)b * ms * D, Xs + (strideXs ? (b0 + b) * strideXs : 0), ms, D, ldxs);
-        if (rc) break;
-        if (cudaMemcpyAsync(dy, y + (size_t)b0 * n, (size_t)bc * n * sizeof(double), cudaMemcpyHostToDevice, h->stream) != cudaSuccess) { rc = GPK_ECUDA; break; }
+        if (!rc) rc = upload_stack(h, dX, X + b0 * strideX, strideX ? bc : 1, n, D, ldx, strideX);
+        if (!rc) rc = upload_stack(h, dXs, Xs + b0 * strideXs, strideXs ? bc : 1, ms, D, ldxs, strideXs);
+        if (rc) return rc;
+        GPK_CUDA(h, cudaMemcpyAsync(dy, y + (size_t)b0 * n, (size_t)bc * n * sizeof(double), cudaMemcpyHostToDevice, h->stream));
         const int64_t sX = strideX ? (int64_t)n * D : 0, sXs = strideXs ? (int64_t)ms * D : 0;
         rc = fit_core(h, w, bc, dX, n, D, n, sX, dy, pp0, 0, w.Li, w.alpha, dll, 1, w.info_dev);
-        if (rc) break;
+        if (rc) return rc;
         // predictions use the kernel without the Option sigmaNoise: extra_diag does not enter cross-covariances
         rc = gpk_posterior(h, dX, n, n, dXs, ms, w.Li, w.alpha, N, pp0.cp, dKsT, dMean, dV, ms, dVar, bc, sX, sXs,
                            bc > 1 ? w.pp_dev : nullptr);
-        if (rc) break;
-        cudaError_t e = cudaMemcpy2DAsync(mean + (size_t)b0 * ms, (size_t)ms * sizeof(double), dMean, (size_t)M * sizeof(double),
-                                          (size_t)ms * sizeof(double), (size_t)bc, cudaMemcpyDeviceToHost, h->stream);
-        if (e == cudaSuccess) e = cudaMemcpy2DAsync(var + (size_t)b0 * ms, (size_t)ms * sizeof(double), dVar, (size_t)M * sizeof(double),
-                                                    (size_t)ms * sizeof(double), (size_t)bc, cudaMemcpyDeviceToHost, h->stream);
-        if (e == cudaSuccess && ll) e = cudaMemcpyAsync(ll + b0, dll, (size_t)bc * sizeof(double), cudaMemcpyDeviceToHost, h->stream);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(hinfo + b0, w.info_dev, (size_t)bc * sizeof(int), cudaMemcpyDeviceToHost, h->stream);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
-        if (e != cudaSuccess) { rc = gpk_set_error(h, GPK_ECUDA, "batched predict: %s", cudaGetErrorString(e)); break; }
+        if (rc) return rc;
+        GPK_CUDA(h, cudaMemcpy2DAsync(mean + (size_t)b0 * ms, (size_t)ms * sizeof(double), dMean, (size_t)M * sizeof(double),
+                                      (size_t)ms * sizeof(double), (size_t)bc, cudaMemcpyDeviceToHost, h->stream));
+        GPK_CUDA(h, cudaMemcpy2DAsync(var + (size_t)b0 * ms, (size_t)ms * sizeof(double), dVar, (size_t)M * sizeof(double),
+                                      (size_t)ms * sizeof(double), (size_t)bc, cudaMemcpyDeviceToHost, h->stream));
+        if (ll) GPK_CUDA(h, cudaMemcpyAsync(ll + b0, dll, (size_t)bc * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+        rc = fetch_batch_results(h, w.info_dev, 0, bc, info ? info + b0 : nullptr, &failed);
+        if (rc && rc != GPK_ENOTPD) return rc;
         const ProblemParams* hp = (const ProblemParams*)h->pp_host;   // the chunk's records, as stage_params built them
-        for (int b = 0; b < bc; ++b) {
+        for (int b = 0; b < bc; ++b)
             for (int i = 0; i < ms; ++i) var[(size_t)(b0 + b) * ms + i] = gpk_prior_var(hp[b].cp) - var[(size_t)(b0 + b) * ms + i];
-            if (info) info[b0 + b] = hinfo[b0 + b];
-            if (hinfo[b0 + b] && !bad) { bad = 1; h->last_info = hinfo[b0 + b]; }
-        }
     }
-    free(hinfo);
-    if (rc) return rc;
-    if (bad) return gpk_set_error(h, GPK_ENOTPD, "at least one problem of the batch is not positive definite (see info[])");
-    return GPK_OK;
+    return rc;
 }
 
 }  // extern "C"

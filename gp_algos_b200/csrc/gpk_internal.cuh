@@ -74,8 +74,15 @@ int gpk_graph_run(gpk_handle h, int slot, const GraphKey& key, int eager_calls, 
 enum { ARENA_A = 0, ARENA_B = 1, ARENA_T = 2, ARENA_MISC = 3, ARENA_X = 4, ARENA_IO = 5, ARENA_IO2 = 6, ARENA_IO3 = 7, ARENA_PP = 8, ARENA_INFO = 9, ARENA_GEMV = 10, ARENA_KINV = 11, GPK_NARENA = 12 };
 
 int gpk_set_error(gpk_handle h, int status, const char* fmt, ...);
+// The arguments shared by every entry point that takes (X, D, theta): a handle, n >= n_min rows, ldx >= n,
+// 1 <= D <= GPK_MAX_D and 0 <= nparams <= gpk_theta_len(h, D) (0 where the entry point computes no gradient).  `ok` carries
+// the entry point's own conditions.  GPK_EINVAL with one message naming `fn`; runs before anything is sized from D.
+int gpk_check_args(gpk_handle h, const char* fn, bool ok, int n, int n_min, int64_t ldx, int D, int nparams);
 // returns device pointer to at least `bytes` bytes in arena `which` (contents undefined after growth)
 void* gpk_arena(gpk_handle h, int which, size_t bytes);
+#define ARENA_OR_FAIL(ptr, type, h, which, bytes)           \
+    type ptr = (type)gpk_arena((h), (which), (bytes));      \
+    if (!ptr) return GPK_ENOMEM
 int gpk_upload_matrix(gpk_handle h, double* dst, const double* src, int rows, int cols, int64_t ld);   // host (ld) -> device (ld = rows)
 int gpk_download_matrix(gpk_handle h, double* dst, int64_t ld, const double* src, int rows, int cols);  // device (ld = rows) -> host (ld)
 int gpk_finish_info(gpk_handle h);  // sync, read h->d_info[0], map to GPK_ENOTPD
@@ -197,6 +204,7 @@ struct ProblemParams {
     CovParams cp;
     double gscale[GPK_MAX_D + 2];  // 1/2 * {2 sf, sf^2 / l_d^3 ..., 2 sn}: factors of the gradient trace
 };
+// D has passed gpk_check_args
 int gpk_make_cov_params(gpk_handle h, const double* theta, int D, int has_sigma_noise, double sigma_noise, CovParams* out);
 int gpk_make_problem_params(gpk_handle h, const double* theta, int D, int has_sigma_noise, double sigma_noise, ProblemParams* out);
 
@@ -270,8 +278,8 @@ int gpk_potrf_factor_solve(gpk_handle h, double* A, double* Li, double* T, int N
 int gpk_potrf_factor(gpk_handle h, double* A, double* Li, double* T, int N, int* info_dev);
 // X = Lw^-1 B (backward == 0) or Lw^-t B (backward != 0) by blocked substitution on the padded lower factor Lw (N x N, ld N).
 // Di: N x 128 scratch for the inverses of the diagonal blocks.  M > 0: B, X are N x M (ld N, M a multiple of 128);
-// M == 0: one vector.  B is overwritten.
-int gpk_trsm_padded(gpk_handle h, const double* Lw, double* Di, int N, int backward, double* B, double* X, int M);
+// M == 0: nvec vectors (ld N), each solved by mat-vecs.  B is overwritten.
+int gpk_trsm_padded(gpk_handle h, const double* Lw, double* Di, int N, int backward, double* B, double* X, int M, int nvec = 1);
 // L^-1 for a given lower-triangular L (N x N padded, ld N)
 int gpk_trtri_lower(gpk_handle h, const double* L, double* Li, double* T, int N);
 // Kinv (lower triangle incl. diagonal tiles in full) = Li^t Li
@@ -310,9 +318,19 @@ size_t gpk_grad_scratch_doubles(int N, int D);
 int gpk_copy2d(gpk_handle h, double* dst, int64_t ldd, const double* src, int64_t lds, int rows, int cols);
 // dst[b*N + i] = i < n ? src[b*n + i] : 0
 int gpk_pad_vector(gpk_handle h, double* dst, int N, const double* src, int n, int batch = 1);
-// dst (N x N padded, lower + identity padding) from src (n x n, ld lds); optionally checks symmetry -> d_flag
-int gpk_load_sym_padded(gpk_handle h, double* dst, int N, const double* src, int n, int64_t lds, int* d_notsym);
-// dst (n x n, ld) = lower triangle of src (N x N) with zeros above the diagonal
-int gpk_store_lower(gpk_handle h, double* dst, int64_t ldd, const double* src, int N, int n);
+// How a square n x n matrix fills a padded N x N one (ld N)
+enum {
+    GPK_PAD_SYM,     // lower triangle and full diagonal 128-blocks of a symmetric matrix, identity padding
+    GPK_PAD_LOWER,   // lower triangle, zeros above the diagonal, identity padding
+    GPK_PAD_UPPER,   // the upper triangle read as its transpose (the lower factor of src^t), identity padding
+    GPK_PAD_FULL     // every entry, zero padding
+};
+// dst (N x N) from the device matrix src (n x n, ld lds) in one launch; GPK_PAD_SYM with d_notsym: *d_notsym = 1 when src is
+// not symmetric
+int gpk_load_padded(gpk_handle h, double* dst, int N, const double* src, int n, int64_t lds, int form, int* d_notsym = nullptr);
+// the same from a host matrix, staged through ARENA_IO (n*n doubles)
+int gpk_upload_padded(gpk_handle h, double* dst, int N, const double* src, int n, int64_t lds, int form, int* d_notsym = nullptr);
+// device dst (n x n, ld ldd) = lower triangle of the padded src (N x N) with zeros above the diagonal, or its transpose
 int gpk_store_tri(gpk_handle h, double* dst, int64_t ldd, const double* src, int N, int n, int transpose);
-int gpk_load_tri_padded(gpk_handle h, double* dst, int N, const double* src, int n, int64_t lds, int transpose_in);
+// the same into a host matrix, staged through ARENA_IO (n*n doubles); dst is written once the stream is synchronised
+int gpk_download_tri(gpk_handle h, double* dst, int64_t ldd, const double* src, int N, int n, int transpose);

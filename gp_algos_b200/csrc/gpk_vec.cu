@@ -194,6 +194,13 @@ __global__ void load_tri_padded_kernel(double* dst, int N, const double* src, in
     dst[r + (int64_t)c * N] = v;
 }
 
+// dst (N x N) = src (n x n, ld) zero padded
+__global__ void load_full_padded_kernel(double* dst, int N, const double* src, int n, int64_t lds) {
+    const int r = blockIdx.y * blockDim.x + threadIdx.x, c = blockIdx.x;
+    if (r >= N) return;
+    dst[r + (int64_t)c * N] = (r < n && c < n) ? src[r + (int64_t)c * lds] : 0.0;
+}
+
 // dst (n x n, ld) = tri(src): lower triangle of src (transpose == 0) or its transpose into the upper triangle
 __global__ void store_tri_kernel(double* dst, int64_t ldd, const double* src, int N, int n, int transpose) {
     const int r = blockIdx.y * blockDim.x + threadIdx.x, c = blockIdx.x;
@@ -292,14 +299,11 @@ int gpk_pad_vector(gpk_handle h, double* dst, int N, const double* src, int n, i
     return GPK_OK;
 }
 
-int gpk_load_sym_padded(gpk_handle h, double* dst, int N, const double* src, int n, int64_t lds, int* d_notsym) {
-    load_sym_padded_kernel<<<dim3(N, (N + 127) / 128), 128, 0, h->stream>>>(dst, N, src, n, lds, d_notsym);
-    GPK_LAUNCH_CHECK(h);
-    return GPK_OK;
-}
-
-int gpk_load_tri_padded(gpk_handle h, double* dst, int N, const double* src, int n, int64_t lds, int transpose_in) {
-    load_tri_padded_kernel<<<dim3(N, (N + 127) / 128), 128, 0, h->stream>>>(dst, N, src, n, lds, transpose_in);
+int gpk_load_padded(gpk_handle h, double* dst, int N, const double* src, int n, int64_t lds, int form, int* d_notsym) {
+    const dim3 grid(N, (N + 127) / 128);
+    if (form == GPK_PAD_SYM) load_sym_padded_kernel<<<grid, 128, 0, h->stream>>>(dst, N, src, n, lds, d_notsym);
+    else if (form == GPK_PAD_FULL) load_full_padded_kernel<<<grid, 128, 0, h->stream>>>(dst, N, src, n, lds);
+    else load_tri_padded_kernel<<<grid, 128, 0, h->stream>>>(dst, N, src, n, lds, form == GPK_PAD_UPPER);
     GPK_LAUNCH_CHECK(h);
     return GPK_OK;
 }
@@ -309,8 +313,4 @@ int gpk_store_tri(gpk_handle h, double* dst, int64_t ldd, const double* src, int
     store_tri_kernel<<<dim3(n, (n + 127) / 128), 128, 0, h->stream>>>(dst, ldd, src, N, n, transpose);
     GPK_LAUNCH_CHECK(h);
     return GPK_OK;
-}
-
-int gpk_store_lower(gpk_handle h, double* dst, int64_t ldd, const double* src, int N, int n) {
-    return gpk_store_tri(h, dst, ldd, src, N, n, 0);
 }
