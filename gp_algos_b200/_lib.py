@@ -110,6 +110,11 @@ def load():
         lib.gpk_debug_ep_site_timing.argtypes = [vp, C.c_int, vp]
         lib.gpk_debug_gemm.argtypes = [vp, vp, _i64, _i64, vp, _i64, _i64, vp, _i64, _i64, vp, _i64, _i64,
                                        ci, ci, ci, ci, cd, cd, ci, ci, ci]
+        lib.gpk_debug_cov.argtypes = [vp, ci, vp, ci, _i64, vp, ci, _i64, ci, vp, ci, cd, vp, _i64, ci, ci, ci, _i64, _i64, _i64]
+        lib.gpk_debug_grad_trace.argtypes = [vp, vp, ci, vp, ci, ci, _i64, vp, vp, ci, vp, ci, _i64, _i64]
+        lib.gpk_debug_trmv.argtypes = [vp, ci, vp, ci, vp, vp, ci]
+        lib.gpk_debug_colwise_dot.argtypes = [vp, vp, _i64, ci, ci, vp, vp, ci, ci, _i64, _i64, _i64]
+        lib.gpk_debug_loglik.argtypes = [vp, vp, ci, ci, vp, vp, vp, ci, _i64]
         lib.gpk_mg_create.argtypes = [C.POINTER(vp), ci, vp]
         lib.gpk_mg_destroy.argtypes = [vp]
         lib.gpk_mg_last_error.argtypes = [vp]

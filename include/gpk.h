@@ -75,6 +75,31 @@ enum { GPK_GEMM_TRI_OUT = 1, GPK_GEMM_KB_R = 2, GPK_GEMM_KB_S = 4, GPK_GEMM_KE_R
 int gpk_debug_gemm(gpk_handle h, const double* P, int64_t ldp, int64_t strideP, const double* Q, int64_t ldq, int64_t strideQ,
                    double* D, int64_t ldd, int64_t strideD, const double* Cin, int64_t ldc, int64_t strideC, int R, int S, int K,
                    int batch, double alpha, double beta, int p_kcontig, int q_kcontig, int flags);
+/* Development aids, not part of the drop-in surface (tests/test_gpu_eval_kernels.py): each runs one internal routine of the
+ * evaluation once, on device pointers, asynchronously on the handle's stream, and returns its status.  Hyper-parameters are
+ * HOST arrays of `batch` theta vectors of the handle's kernel family, back to back; problem b reads X at + b*strideX.
+ * gpk_debug_cov: the covariance build of the handle's family.
+ *   SYM_FULL       K (m x m, ld ldk) = k(X1, X1) + (sn^2 + sigma_noise) I, lower 64-tiles computed and mirrored; batch 1.
+ *   SYM_LOWER_PAD  K (mp x mp, ld mp, problem b at + b*mp*mp; mp a multiple of 128 and >= m): every 64-tile whose 128-block
+ *                  is on or below the diagonal, with identity padding beyond m; the 128-blocks above it are not written.
+ *   CROSS          K (ld ldk, at + b*strideK) = k(X1, X2) without noise, zero-filled up to (mp, np); nothing beyond.
+ * gpk_debug_grad_trace: g[b*strideOut + p] = 1/2 sum_{i,j<n} (alpha_i alpha_j - Kinv_ij) dk_p(x_i, x_j) for p < nparams, reading
+ *   the lower 64-tiles of Kinv (N x N at + b*N*N; NULL: alpha alpha^t alone) and alpha (at + b*N).
+ * gpk_debug_trmv: out = Li x (transposed == 0) or Li^t x, Li N x N lower (at + b*N*N), x and out at + b*N.
+ * gpk_debug_colwise_dot: out[b*strideOut + c] = sum_{r<rows} M[b*strideM + r + c*ld] * (square ? M[..] : v[b*strideV + r]).
+ * gpk_debug_loglik: out[b*strideOut] = -1/2 y.alpha - sum_{i<n} log A_ii - n/2 log(2 pi), A N x N at + b*N*N, y, alpha at + b*N. */
+enum { GPK_DEBUG_COV_SYM_FULL = 0, GPK_DEBUG_COV_SYM_LOWER_PAD = 1, GPK_DEBUG_COV_CROSS = 2 };
+int gpk_debug_cov(gpk_handle h, int mode, const double* dX1, int m, int64_t ldx1, const double* dX2, int n, int64_t ldx2, int D,
+                  const double* thetas_host, int has_sigma_noise, double sigma_noise, double* dK, int64_t ldk, int mp, int np,
+                  int batch, int64_t strideX1, int64_t strideX2, int64_t strideK);
+int gpk_debug_grad_trace(gpk_handle h, const double* dKinv, int N, const double* dX, int n, int D, int64_t ldx,
+                         const double* dalpha, const double* thetas_host, int nparams, double* dg, int batch, int64_t strideX,
+                         int64_t strideOut);
+int gpk_debug_trmv(gpk_handle h, int transposed, const double* dLi, int N, const double* dx, double* dout, int batch);
+int gpk_debug_colwise_dot(gpk_handle h, const double* dM, int64_t ld, int rows, int cols, const double* dv, double* dout,
+                          int square, int batch, int64_t strideM, int64_t strideV, int64_t strideOut);
+int gpk_debug_loglik(gpk_handle h, const double* dA, int N, int n, const double* dy, const double* dalpha, double* dout,
+                     int batch, int64_t strideOut);
 /* Launch sequences that callers repeat verbatim are captured into CUDA graphs and replayed: the single-problem
  * gpk_gp_nll_grad[_dev] evaluation (an optimiser's objective, GpPredictor.scala:126-142; same buffers and shape, new
  * hyper-parameters through device memory) from its second call on, the device-resident factor-only Cholesky up to n = 4096
