@@ -108,6 +108,11 @@ def load():
         lib.gpk_gp_predict_batched.argtypes = [vp, ci, vp, ci, ci, _i64, _i64, vp, vp, vp, ci, _i64, _i64, ci, cd, vp, vp, vp, vp]
         lib.gpk_debug_base_timing.argtypes = [vp, vp]
         lib.gpk_debug_ep_site_timing.argtypes = [vp, C.c_int, vp]
+        lib.gpk_debug_ep_scalar.argtypes = [vp, ci, vp, ci, vp]
+        lib.gpk_debug_ep_sites.argtypes = [vp, ci, vp, ci, ci, vp, vp, vp, vp, vp, vp, vp, vp]
+        lib.gpk_debug_ep_apply.argtypes = [vp, vp, ci, ci, ci, ci, vp, vp, vp, vp, vp, vp]
+        lib.gpk_debug_ep_site_loop.argtypes = [vp, vp, ci, vp, vp, vp, vp, vp, vp, vp, vp, vp]
+        lib.gpk_debug_ep_refactor.argtypes = [vp, vp, ci, vp, vp, vp, vp, vp]
         lib.gpk_debug_gemm.argtypes = [vp, vp, _i64, _i64, vp, _i64, _i64, vp, _i64, _i64, vp, _i64, _i64,
                                        ci, ci, ci, ci, cd, cd, ci, ci, ci]
         lib.gpk_debug_cov.argtypes = [vp, ci, vp, ci, _i64, vp, ci, _i64, ci, vp, ci, cd, vp, _i64, ci, ci, ci, _i64, _i64, _i64]

@@ -62,6 +62,39 @@ int gpk_debug_base_timing(gpk_handle h, long long* stamps_host);
  * one unstamped launch of the default kernel, [321..576] barrier arrival of four other warps per site, [577..896] phases of
  * tile warp 0 (the last two groups for chain >= 10 only). */
 int gpk_debug_ep_site_timing(gpk_handle h, int chain, long long* stamps_host);
+/* Development aids, not part of the drop-in surface (tests/test_gpu_ep_kernels.py): each issues exactly one routine of the EP
+ * sweep (csrc/gpk_ep.cu) on device pointers, asynchronously on the handle's stream, and returns its status.
+ * gpk_debug_ep_scalar: one scalar primitive of the site kernels per element, c_erfcx staged in shared memory as the site kernel
+ *   stages it.  Per element i:
+ *     RCP, EXP_NEG_SQ, ERFCX_TAB, RATIO, RATIO_FAST   in[i] -> out[i]   (rcp_nr, exp_neg_sq, erfcx_tab, dnorm_over_pnorm,
+ *                                                                        dnorm_over_pnorm_fast)
+ *     RSQRT        in[i] -> out[2i] = rsqrt_nr, out[2i+1] = libdevice rsqrt
+ *     SITE_FAST    in[5i..] = (sii, mui, t_old, n_old, y) -> out[9i..] = (c, g, mu_hat, sig_hat, rs, ct, cn, tau, nu) of
+ *                  ep_site_fast, tau and nu finished as ep_sites_block_p finishes them
+ *     SITE_SCALAR  in[5i..] as above -> out[6i..] = (ct, cn, c, g, dtau, nu) of ep_site_scalar
+ * gpk_debug_ep_sites: one launch of the site kernel (variant 5: ep_sites_block_p, 4: ep_sites_block_w) on the 64 x 64 block Dg
+ *   (column-major; the leading bsz x bsz is read) for the sites i0 .. i0+bsz-1 of mu, tau, nu, cav_tau, cav_nu and y; writes
+ *   blk = (c[64], g[64]) and W = (I + A)^-1 (64 x 64 column-major).
+ * gpk_debug_ep_apply: one launch of ep_apply_gemm for block b (bsz sites) of an n-site sweep: Sigma0 N x N (lower triangle
+ *   outside tile (b, b)), Dg the N/64 diagonal 64 x 64 blocks, U and P N x 64 (ld N), mu N.
+ * gpk_debug_ep_site_loop: the site loop of one sweep (site kernel, apply and delayed flush of every block; variant from
+ *   GPK_EP_SITES) from Sigma0 (N x N lower, N = n rounded up to a multiple of 128) and the n-vectors tau, nu, mu, y; writes the
+ *   n-vectors tau, nu, mu, cav_tau, cav_nu after the sweep.
+ * gpk_debug_ep_refactor: the posterior re-factorisation from K (n x n, ld n) and the n-vectors tau, nu: L = chol(I + S^1/2 K S^1/2)
+ *   and Sigma = K - V^t V (N x N, ld N, lower tiles), mu = Sigma nu (n); waits for the result and returns GPK_ENOTPD if B
+ *   is not positive definite. */
+enum { GPK_DEBUG_EP_RCP = 0, GPK_DEBUG_EP_RSQRT = 1, GPK_DEBUG_EP_EXP_NEG_SQ = 2, GPK_DEBUG_EP_ERFCX_TAB = 3, GPK_DEBUG_EP_RATIO = 4,
+       GPK_DEBUG_EP_RATIO_FAST = 5, GPK_DEBUG_EP_SITE_FAST = 6, GPK_DEBUG_EP_SITE_SCALAR = 7 };
+int gpk_debug_ep_scalar(gpk_handle h, int what, const double* d_in, int count, double* d_out);
+int gpk_debug_ep_sites(gpk_handle h, int variant, const double* dDg, int i0, int bsz, const double* dmu, double* dtau, double* dnu,
+                       double* dcav_tau, double* dcav_nu, const int* dy, double* dblk, double* dW);
+int gpk_debug_ep_apply(gpk_handle h, const double* dSigma0, int N, int n, int b, int bsz, const double* dblk, const double* dW,
+                       double* dU, double* dP, double* dmu, double* dDg);
+int gpk_debug_ep_site_loop(gpk_handle h, const double* dSigma0, int n, const double* dtau, const double* dnu, const double* dmu,
+                           const int* dy, double* dtau_out, double* dnu_out, double* dmu_out, double* dcav_tau_out,
+                           double* dcav_nu_out);
+int gpk_debug_ep_refactor(gpk_handle h, const double* dK, int n, const double* dtau, const double* dnu, double* dL, double* dSigma,
+                          double* dmu);
 /* Development aid, not part of the drop-in surface (tests/test_gpu_gemm.py): issues exactly one internal DMMA GEMM with the
  * descriptor given field by field and returns its status (GPK_EINVAL, without a launch, for R or S not a multiple of 64, K not
  * a multiple of 16, an odd leading dimension or a pointer that is not 16-byte aligned).  Device pointers; for every 64 x 64
