@@ -33,7 +33,8 @@ from . import batched  # noqa: F401
 from .ep_classification import (EpParameterEstimator, GpClassifier, MarginalLikelihoodEvaluator, SiteParams,  # noqa: F401
                                 AvgBasedStopCriterion, FixedSweeps, ClassifierInput, AfterEstimationClassifierInput,
                                 HyperParameterOptimInput, GradientHyperParamsOptimizer, ApacheCommonsOptimizer,
-                                MeshHyperParamsLogLikelihoodEvaluator, HyperParamsMeshValues)
+                                MeshHyperParamsLogLikelihoodEvaluator, HyperParamsMeshValues, log_likelihood_batched,
+                                obtain_optimal_ep_hyper_params_multistart)
 from .gp_optimizer import GPOptimizer, GPOInput, BreezeLbfgsOptimizer, ucb_with_gradient  # noqa: F401
 from .gp_ukf import (GPUnscentedKalmanFilter, UnscentedTransformParams, UnscentedFilteringInput, SsmModel,  # noqa: F401
                      FilteringOutput)

@@ -102,6 +102,8 @@ def load():
         lib.gpk_ep_fit.argtypes = [vp, vp, ci, _i64, vp, cd, ci, ci, ci, vp, vp, vp, vp, _i64, vp, vp, vp, vp]
         lib.gpk_ep_classify.argtypes = [vp, vp, ci, _i64, vp, ci, _i64, vp, vp, vp, vp, _i64, vp, vp, vp]
         lib.gpk_ep_nll_grad.argtypes = [vp, vp, ci, ci, _i64, vp, vp, cd, ci, ci, ci, ci, vp, vp, vp, vp, vp]
+        lib.gpk_ep_nll_grad_batched.argtypes = [vp, ci, vp, ci, ci, _i64, _i64, vp, vp, _i64, cd, ci, ci, ci, ci, vp, vp, vp, vp,
+                                                vp, vp]
         lib.gpk_ep_grad_from_factor.argtypes = [vp, vp, ci, ci, _i64, vp, vp, _i64, vp, vp, vp, _i64, ci, vp]
         lib.gpk_gp_nll_grad_batched.argtypes = [vp, ci, vp, ci, ci, _i64, _i64, vp, vp, ci, cd, ci, vp, vp, vp]
         lib.gpk_gp_nll_grad_batched_dev.argtypes = [vp, ci, vp, ci, ci, _i64, _i64, vp, vp, ci, cd, ci, vp, vp]

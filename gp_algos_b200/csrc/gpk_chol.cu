@@ -529,8 +529,8 @@ int gpk_potrf_factor_solve(gpk_handle h, double* A, double* Li, double* T, int N
 
 bool gpk_use_pipelined(int N, int batch) { return batch == 1 && pipe_min() > 0 && N >= pipe_min() && N >= 2 * pipe_nb(); }
 
-int gpk_potrf_inv(gpk_handle h, double* A, double* Li, double* T, int N, int keep_L, int* info_dev, int batch) {
-    if (gpk_use_pipelined(N, batch)) return gpk_potrf_inv_pipelined(h, A, Li, nullptr, T, N, keep_L, info_dev, nullptr);
+int gpk_potrf_inv(gpk_handle h, double* A, double* Li, double* T, int N, int keep_L, int* info_dev, int batch, bool lookahead) {
+    if (lookahead && gpk_use_pipelined(N, batch)) return gpk_potrf_inv_pipelined(h, A, Li, nullptr, T, N, keep_L, info_dev, nullptr);
     GPK_CUDA(h, cudaMemsetAsync(info_dev, 0, sizeof(int) * (size_t)batch, h->stream));
     const int64_t sM = (int64_t)N * N, sT = (int64_t)gpk_chol_scratch_doubles(N);
     if (batch < 8) {

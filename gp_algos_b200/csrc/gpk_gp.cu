@@ -13,15 +13,6 @@
 
 namespace {
 
-size_t batch_budget_bytes() {
-    static size_t v = 0;
-    if (!v) {
-        const char* e = getenv("GPK_BATCH_GB");
-        v = (size_t)((e ? atof(e) : 48.0) * (1ull << 30));
-    }
-    return v;
-}
-
 // Per-problem working set of the fused pipelines.
 struct Work {
     int N, B;          // padded size, problems resident at once
@@ -141,41 +132,6 @@ int nll_grad_core(gpk_handle h, int B, const double* dX, int n, int D, int64_t l
             if (rc) return rc;
         }
     }
-    return GPK_OK;
-}
-
-// A stack of nx host matrices (n x D, ld ldx, matrix b at X + b*stride) to the device, compact and back to back (matrix b at
-// dst + b*n*D): one copy when the stack already is laid out so (Breeze matrices back to back)
-int upload_stack(gpk_handle h, double* dst, const double* X, int nx, int n, int D, int64_t ldx, int64_t stride) {
-    if (ldx == n && (nx == 1 || stride == (int64_t)n * D)) {
-        GPK_CUDA(h, cudaMemcpyAsync(dst, X, (size_t)nx * n * D * sizeof(double), cudaMemcpyHostToDevice, h->stream));
-        return GPK_OK;
-    }
-    int rc = GPK_OK;
-    for (int b = 0; b < nx && !rc; ++b) rc = gpk_upload_matrix(h, dst + (size_t)b * n * D, X + b * stride, n, D, ldx);
-    return rc;
-}
-
-// The results of a batched call come back through the handle's pinned staging (grown on demand, never per call): res_bytes
-// of results at dres (0: none) followed on the device by the B per-problem info words, staged at h->res_pinned in one copy
-// and one synchronisation.  info (optional) receives the info words.  The call's first failure goes to h->last_info and
-// sets *failed, which stays set across the chunks of one call: GPK_ENOTPD from then on.
-int fetch_batch_results(gpk_handle h, const void* dres, size_t res_bytes, int B, int* info, bool* failed) {
-    const size_t bytes = res_bytes + (size_t)B * sizeof(int);
-    if (h->res_pinned_bytes < bytes) {
-        if (h->res_pinned) cudaFreeHost(h->res_pinned);
-        h->res_pinned = nullptr; h->res_pinned_bytes = 0;
-        if (cudaMallocHost(&h->res_pinned, bytes) != cudaSuccess) { cudaGetLastError(); return gpk_set_error(h, GPK_ENOMEM, "pinned host allocation failed"); }
-        h->res_pinned_bytes = bytes;
-    }
-    GPK_CUDA(h, cudaMemcpyAsync(h->res_pinned, dres, bytes, cudaMemcpyDeviceToHost, h->stream));
-    GPK_CUDA(h, cudaStreamSynchronize(h->stream));
-    const int* hinfo = (const int*)((const char*)h->res_pinned + res_bytes);
-    for (int b = 0; b < B; ++b) {
-        if (info) info[b] = hinfo[b];
-        if (hinfo[b] && !*failed) { *failed = true; h->last_info = hinfo[b]; }
-    }
-    if (*failed) return gpk_set_error(h, GPK_ENOTPD, "at least one problem of the batch is not positive definite (see info[])");
     return GPK_OK;
 }
 
@@ -338,6 +294,50 @@ int gpk_posterior(gpk_handle h, const double* dX, int n, int64_t ldx, const doub
     rc = gpk_trmm_lower(h, Li, N, KsT, V, gpk_pad(nv), batch);                                                     // :55
     if (rc || !vsq) return rc;
     return gpk_colwise_dot(h, V, N, N, nv, nullptr, vsq, 1, batch, sK, 0, M);                                      // :56, diagonal
+}
+
+size_t batch_budget_bytes() {
+    static size_t v = 0;
+    if (!v) {
+        const char* e = getenv("GPK_BATCH_GB");
+        v = (size_t)((e ? atof(e) : 48.0) * (1ull << 30));
+    }
+    return v;
+}
+
+// A stack of nx host matrices (n x D, ld ldx, matrix b at X + b*stride) to the device, compact and back to back (matrix b at
+// dst + b*n*D): one copy when the stack already is laid out so (Breeze matrices back to back)
+int upload_stack(gpk_handle h, double* dst, const double* X, int nx, int n, int D, int64_t ldx, int64_t stride) {
+    if (ldx == n && (nx == 1 || stride == (int64_t)n * D)) {
+        GPK_CUDA(h, cudaMemcpyAsync(dst, X, (size_t)nx * n * D * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+        return GPK_OK;
+    }
+    int rc = GPK_OK;
+    for (int b = 0; b < nx && !rc; ++b) rc = gpk_upload_matrix(h, dst + (size_t)b * n * D, X + b * stride, n, D, ldx);
+    return rc;
+}
+
+// The results of a batched call come back through the handle's pinned staging (grown on demand, never per call): res_bytes
+// of results at dres (0: none) followed on the device by the B per-problem info words, staged at h->res_pinned in one copy
+// and one synchronisation.  info (optional) receives the info words.  The call's first failure goes to h->last_info and
+// sets *failed, which stays set across the chunks of one call: GPK_ENOTPD from then on.
+int fetch_batch_results(gpk_handle h, const void* dres, size_t res_bytes, int B, int* info, bool* failed) {
+    const size_t bytes = res_bytes + (size_t)B * sizeof(int);
+    if (h->res_pinned_bytes < bytes) {
+        if (h->res_pinned) cudaFreeHost(h->res_pinned);
+        h->res_pinned = nullptr; h->res_pinned_bytes = 0;
+        if (cudaMallocHost(&h->res_pinned, bytes) != cudaSuccess) { cudaGetLastError(); return gpk_set_error(h, GPK_ENOMEM, "pinned host allocation failed"); }
+        h->res_pinned_bytes = bytes;
+    }
+    GPK_CUDA(h, cudaMemcpyAsync(h->res_pinned, dres, bytes, cudaMemcpyDeviceToHost, h->stream));
+    GPK_CUDA(h, cudaStreamSynchronize(h->stream));
+    const int* hinfo = (const int*)((const char*)h->res_pinned + res_bytes);
+    for (int b = 0; b < B; ++b) {
+        if (info) info[b] = hinfo[b];
+        if (hinfo[b] && !*failed) { *failed = true; h->last_info = hinfo[b]; }
+    }
+    if (*failed) return gpk_set_error(h, GPK_ENOTPD, "at least one problem of the batch is not positive definite (see info[])");
+    return GPK_OK;
 }
 
 extern "C" {

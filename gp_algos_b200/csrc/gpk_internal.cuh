@@ -233,6 +233,17 @@ int gpk_posterior(gpk_handle h, const double* dX, int n, int64_t ldx, const doub
                   const double* alpha, int N, const CovParams& cp, double* KsT, double* mean, double* V, int nv, double* vsq,
                   int batch = 1, int64_t strideX = 0, int64_t strideXs = 0, const ProblemParams* pp_dev = nullptr);
 
+// What the batched entry points share (gpk_gp.cu):
+// bytes of device memory one batched call may hold for its problems at once (GPK_BATCH_GB, default 48 GiB); a larger batch
+// runs chunk by chunk
+size_t batch_budget_bytes();
+// nx host matrices (n x D, ld ldx, matrix b at X + b*stride) to the device, back to back at dst + b*n*D
+int upload_stack(gpk_handle h, double* dst, const double* X, int nx, int n, int D, int64_t ldx, int64_t stride);
+// res_bytes of results at dres followed on the device by B info words, through the handle's pinned staging (h->res_pinned)
+// in one copy and one synchronisation; info (optional) receives the info words; *failed is set at the first non-zero one
+// (GPK_ENOTPD from then on, across the chunks of one call)
+int fetch_batch_results(gpk_handle h, const void* dres, size_t res_bytes, int B, int* info, bool* failed);
+
 // ---------------------------------------------------------------------------------------------
 // covariance (gpk_cov.cu)
 // ---------------------------------------------------------------------------------------------
@@ -260,7 +271,10 @@ int gpk_cov_deriv(gpk_handle h, int param_num, const double* dX, int n, int64_t 
 int gpk_base_potrf_trtri(gpk_handle h, double* A, int64_t lda, double* Li, int64_t ldi, int* info, int col_offset, int mode,
                          int batch, int64_t strideA, int64_t strideLi, int info_stride, int coloff_stride);
 size_t gpk_chol_scratch_doubles(int N);
-int gpk_potrf_inv(gpk_handle h, double* A, double* Li, double* T, int N, int keep_L, int* info_dev, int batch = 1);
+// lookahead == false: the recursion for every batch count (a batch of one above GPK_PIPE_MIN included), so that a problem's
+// results do not depend on how many problems share the call
+int gpk_potrf_inv(gpk_handle h, double* A, double* Li, double* T, int N, int keep_L, int* info_dev, int batch = 1,
+                  bool lookahead = true);
 // Look-ahead driver for one large problem (see gpk_chol.cu): same results as gpk_potrf_inv; when Kinv != nullptr it also
 // accumulates K^-1 = Li^t Li (lower tiles) into Kinv (N x N, ld N, a buffer distinct from A and Li).
 bool gpk_use_pipelined(int N, int batch);

@@ -1,5 +1,5 @@
 """Host mirror of gp/classification/{EpParameterEstimator, GpClassifier, MarginalLikelihoodEvaluator}.scala over
-libgpk's EP entry points (gpk_ep_fit, gpk_ep_classify)."""
+libgpk's EP entry points (gpk_ep_fit, gpk_ep_classify, gpk_ep_nll_grad[_batched])."""
 from __future__ import annotations
 
 import ctypes as C
@@ -9,6 +9,7 @@ from typing import Optional
 import numpy as np
 
 from . import _lib
+from . import batched as _batched
 from . import matrix_utils as MU
 
 
@@ -248,6 +249,55 @@ class ApacheCommonsOptimizer:
         except _TooManyEvaluations:
             point = best["x"]
         return init.fromDenseVector(np.asarray(point, dtype=np.float64))
+
+
+def log_likelihood_batched(X, targets, thetas, stopCriterion, nparams: Optional[int] = None, keep_linebreak_quirk: bool = True,
+                           handle=None):
+    """B evaluations of MarginalLikelihoodEvaluator.logLikelihood (MarginalLikelihoodEvaluator.scala:33-66) of one size n in one
+    call (gpk_ep_nll_grad_batched): every problem runs EP to its own stop, all sweeps together on the device.
+    X: (n, D) shared or (B, n, D); targets: (n,) shared or (B, n); thetas: (B, P) in the handle's kernel family.
+    Returns (logZ[B], grad[B, nparams], sweeps[B], info[B]); a problem with info != 0 (not positive definite) has NaN logZ and
+    gradient, the others are valid."""
+    h = handle or _lib.default_handle()
+    thetas = np.ascontiguousarray(np.atleast_2d(thetas), dtype=np.float64)
+    B = thetas.shape[0]
+    Xb, strideX, n, D = _batched._stack_problems(X, B)
+    t = np.ascontiguousarray(targets, dtype=np.int32)
+    if t.ndim == 1:
+        strideT = 0
+    elif t.ndim == 2 and t.shape[0] == B:
+        strideT = n
+    else:
+        raise _lib.IllegalArgumentError(_lib.GPK_EINVAL, "targets must be (n,) or (B, n)")
+    P = h.lib.gpk_theta_length(h.h, D)
+    if t.shape[-1] != n or thetas.shape[1] != P:
+        raise _lib.IllegalArgumentError(_lib.GPK_EINVAL, "requirement failed: shapes of X, targets and hyper-parameters disagree")
+    nparams = P if nparams is None else int(nparams)
+    eps, fixed, mx = _stop_args(stopCriterion)
+    logz = np.empty(B); grad = np.zeros((B, max(nparams, 1))); sweeps = np.zeros(B, dtype=np.int32)
+    info = np.zeros(B, dtype=np.int32)
+    rc = h.lib.gpk_ep_nll_grad_batched(h.h, B, _lib.ptr(Xb), n, D, n, strideX, _lib.ptr(thetas), _lib.ptr(t), strideT, eps, fixed, mx,
+                                       int(keep_linebreak_quirk), nparams, _lib.ptr(logz), _lib.ptr(grad), None, None,
+                                       _lib.ptr(sweeps), _lib.ptr(info))
+    if rc != _lib.GPK_ENOTPD:
+        h.check(rc)
+    return logz, grad[:, :nparams], sweeps, info
+
+
+def obtain_optimal_ep_hyper_params_multistart(trainData, targets, initThetas, stopCriterion, maxIter: int = 20, handle=None):
+    """GradientHyperParamsOptimizer (HyperParamsOptimization.scala:31-55) from R start points at once: the restarts share the
+    training set and every lockstep round of batched.LockstepLbfgs is ONE gpk_ep_nll_grad_batched call.  The classification
+    twin of batched.obtain_optimal_hyper_params_multistart.  Returns (thetas[R, P], logZ[R]) -- the best-seen point and value
+    of every restart; a restart that never had a positive definite evaluation comes back as its start point with logZ = -inf."""
+    X = np.asarray(trainData, dtype=np.float64)
+    t = np.ascontiguousarray(targets, dtype=np.int32)
+    init = np.atleast_2d(np.asarray(initThetas, dtype=np.float64))
+
+    def objective(points, which):
+        logz, grad, _, info = log_likelihood_batched(X, t, points, stopCriterion, handle=handle)
+        return np.where(info == 0, logz, -np.inf), grad
+
+    return _batched.LockstepLbfgs(maxIter=maxIter).maximize(objective, init)
 
 
 class HyperParamsMeshValues:

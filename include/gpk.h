@@ -139,7 +139,7 @@ int gpk_debug_loglik(gpk_handle h, const double* dA, int N, int n, const double*
  * when the same buffers are factored again, and -- only with GPK_GRAPH_AFTER_EP=k in the environment, after k eager sweeps of one
  * size -- the EP sweep (EpParameterEstimator.scala:37-67; measured slower than eager launches since the round-2 rework).  on = 0: eager launches only; 1 (default,
  * or the GPK_GRAPH environment variable): as described; 2: capture at the first repetition of anything.  Results are
- * bit-identical in every mode. */
+ * bit-identical in every mode.  The batched EP evaluation (gpk_ep_nll_grad_batched) always launches eagerly. */
 int gpk_set_graph_mode(gpk_handle h, int on);
 
 /* ---- kernel family -------------------------------------------------------------------------------
@@ -394,6 +394,21 @@ int gpk_ep_classify(gpk_handle h, const double* K, int n, int64_t ldk, const dou
 int gpk_ep_nll_grad(gpk_handle h, const double* X, int n, int D, int64_t ldx, const double* theta, const int* targets,
                     double eps, int fixed_sweeps, int max_sweeps, int keep_linebreak_quirk, int nparams, double* logZ,
                     double* grad, double* tau, double* nu, int* sweeps);
+/* B evaluations of MarginalLikelihoodEvaluator.logLikelihood (MarginalLikelihoodEvaluator.scala:33-66) of one size n in one
+ * call: the hyper-parameter mesh (MeshHyperParamsLogLikelihoodEvaluator.scala:12-45) and optimiser restarts
+ * (HyperParamsOptimization.scala:31-136) evaluate many points on one training set.  Problem b: X + b*strideX (strideX == 0:
+ * every problem shares X), targets + b*strideT (strideT == 0: shared labels), thetas + b*gpk_theta_length(h, D), the
+ * handle's kernel family.  Stop rule, quirk and nparams exactly as gpk_ep_nll_grad, applied to EACH problem on its own:
+ * each problem stops at its own sweep.  Outputs: logZ[b], grad[b*nparams + p], tau / nu[b*n + i] (may be NULL),
+ * sweeps[b], info[b] (0 or the failing leading minor of I + S^1/2 K S^1/2; may be NULL).  GPK_ENOTPD if any problem
+ * failed (its logZ and gradient are NaN); the others are valid.  nparams == 0: no gradient (logLikelihoodWithoutGrad,
+ * :24-31).  The sweeps of all problems run together (one site-kernel CTA per problem, every other launch batched); a
+ * problem's results do not depend on the other problems of the call or on its position.  Eager launches only:
+ * gpk_set_graph_mode does not apply.  A batch larger than GPK_BATCH_GB (see gpk_gp_nll_grad_batched) runs chunk by chunk. */
+int gpk_ep_nll_grad_batched(gpk_handle h, int B, const double* X, int n, int D, int64_t ldx, int64_t strideX,
+                            const double* thetas, const int* targets, int64_t strideT, double eps, int fixed_sweeps,
+                            int max_sweeps, int keep_linebreak_quirk, int nparams, double* logZ, double* grad,
+                            double* tau, double* nu, int* sweeps, int* info);
 /* MarginalLikelihoodEvaluator.scala:47-66 logLikelihoodDerivativesAfterHyperParams(HyperParameterOptimInput(siteParams,
  * lowerTriangular, kernelMatrix, trainInput), kernelFun): the gradient alone from a finished EP run.  K may be NULL
  * (rebuilt from X and theta). */
